@@ -8,7 +8,7 @@ that 50k x 50k pair matrix (global Gotoh alignment with Biopython's first-path t
 four distance metrics per pair).  With N GPUs under torchrun every rank takes its own tile per
 step (static tile assignment, weak scaling, no collective on the compute path).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python bench.py --config C2|C4|C5 [--gpus N] ...      (one process drives N GPUs)
 
 Prints ONE JSON line (rank 0):
@@ -24,6 +24,8 @@ Prints ONE JSON line (rank 0):
             sensitive pairs re-aligned), checked against the ordinary path on a band of rows
 `--impl reference` times the CPU restatement of the reference path (oracle/, "port": Biopython
 and the Rust distance crate are not installable here) on all host threads, on the same tiles.
+`--dump-outputs DIR` (C3) writes the results of the last timed step (rank 0's tile) as DIR/counts.npy
+and DIR/metrics.npy, for comparing two builds output for output (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -41,6 +43,7 @@ import numpy as np
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests"))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (no __pycache__)
 
 N_SEQ = 50_000
 SEQ_LEN = 650
@@ -48,6 +51,7 @@ TILE_X = 1536
 TILE_Y = 2048
 STRONG_X, STRONG_Y = 8192, 16384
 SYM_N = 8192               # versusAll as a whole job: all ordered pairs of the first SYM_N sequences
+DUMP_PAIRS = 1 << 20       # --dump-outputs: pairs sampled from the last tile (48 MiB; the whole tile is 144 MiB)
 OPS_PER_CELL = 13          # SURVEY.md 8d: scalar INT32 ops of the score-only 3-state recurrence
 SCORES_TEXT = "match 1, mismatch -1, internal open -8 / extend -1, end open -1 / extend -1"
 
@@ -430,6 +434,8 @@ def run_c3(args, rank: int, local_rank: int, world: int) -> None:
     launches = st1["launches"] - st0["launches"]
     kernel_id = eng.last_kernel
     checksum = int(d_counts.sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), d_counts, d_metrics)
 
     # ---- end to end through the C ABI with host buffers ("e2e") --------------------------------
     eng2 = Engine(local_rank)
@@ -524,6 +530,20 @@ def run_c3(args, rank: int, local_rank: int, world: int) -> None:
         print(json.dumps(line), flush=True)
     if distributed:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: Path, d_counts, d_metrics) -> None:
+    """The last timed step's results for a fixed sample of DUMP_PAIRS pairs of its tile (seed 0,
+    in row-major pair order; the same inputs every run): counts.npy (DUMP_PAIRS x 4 {same, ts, tv,
+    gaps} as float32, exact) and metrics.npy (DUMP_PAIRS x 4 {p, p-gaps, jc, k2p} as float64, NaN =
+    undefined)."""
+    import torch
+
+    pick = np.sort(np.random.default_rng(0).choice(d_counts.shape[0], DUMP_PAIRS, replace=False))
+    idx = torch.from_numpy(pick).to(d_counts.device)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "counts.npy", d_counts.index_select(0, idx).float().cpu().numpy())
+    np.save(out_dir / "metrics.npy", d_metrics.index_select(0, idx).cpu().numpy())
 
 
 def trace_bytes(kernel_id: int) -> float:
@@ -804,9 +824,15 @@ def main() -> None:
     ap.add_argument("--nseq", type=int, default=None, help="C3: sequences generated (default 50000); C2: rows (9000); C5: sequences (16384)")
     ap.add_argument("--queries", type=int, default=None, help="C4: queries (default 200000) against 20000 references")
     ap.add_argument("--no-strong", dest="strong", action="store_false", help="C3: skip the fixed-job strong-scaling sub-record")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="C3: write counts.npy and metrics.npy of the last timed step (a seeded sample of its pairs) to DIR")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 5 if args.config in ("C3", "C2") else 1
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.config != "C3" or args.impl != "taxi2_b200"):
+        ap.error("--dump-outputs is implemented for the C3 workload of taxi2_b200 only")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -61,3 +61,29 @@ def best_score(x: str, y: str, scores) -> float:
                 o, e = (eo, ee) if i in (0, nA) else (io, ie)
                 Y[i][j] = max(M[i][j - 1] + o, X[i][j - 1] + o, Y[i][j - 1] + e)
     return max(M[nA][nB], X[nA][nB], Y[nA][nB])
+
+
+def best_score_adjacent_gaps(x: str, y: str, scores) -> float:
+    """max over the global alignments that put a vertical gap right next to a horizontal one (at
+    least one Ix <-> Iy transition); -inf if there is none.  The packed kernel's recurrence drops
+    those transitions, which is exact for a pair iff this stays strictly below best_score."""
+    match, mismatch, io, ie, eo, ee = (float(s) for s in scores)
+    nA, nB = len(x), len(y)
+    # layer 0: no Ix <-> Iy transition yet, layer 1: at least one
+    M = [[[NEG] * (nB + 1) for _ in range(nA + 1)] for _ in range(2)]
+    X = [[[NEG] * (nB + 1) for _ in range(nA + 1)] for _ in range(2)]
+    Y = [[[NEG] * (nB + 1) for _ in range(nA + 1)] for _ in range(2)]
+    M[0][0][0] = 0.0
+    for i in range(nA + 1):
+        for j in range(nB + 1):
+            for k in (0, 1):
+                if i > 0 and j > 0:
+                    s = match if x[i - 1] == y[j - 1] else mismatch
+                    M[k][i][j] = max(M[k][i - 1][j - 1], X[k][i - 1][j - 1], Y[k][i - 1][j - 1]) + s
+                if i > 0:
+                    o, e = (eo, ee) if j in (0, nB) else (io, ie)
+                    X[k][i][j] = max(M[k][i - 1][j] + o, X[k][i - 1][j] + e, Y[1][i - 1][j] + o if k else NEG, Y[0][i - 1][j] + o if k else NEG)
+                if j > 0:
+                    o, e = (eo, ee) if i in (0, nA) else (io, ie)
+                    Y[k][i][j] = max(M[k][i][j - 1] + o, Y[k][i][j - 1] + e, X[1][i][j - 1] + o if k else NEG, X[0][i][j - 1] + o if k else NEG)
+    return max(M[1][nA][nB], X[1][nA][nB], Y[1][nA][nB])

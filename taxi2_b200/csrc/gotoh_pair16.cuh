@@ -23,6 +23,8 @@
 //
 // Rows = x (<= 32*H, single stripe), lane l owns rows [l*H, l*H+H); columns stream one per step.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace taxi {
@@ -68,16 +70,21 @@ __device__ __forceinline__ uint32_t lop3_and_or(uint32_t a, uint32_t mask, uint3
     return r;
 }
 
+// Row symbol codes of the two pairs as diag_candidate() wants them: (-code) mod 2^16 per half
+// (low half = pair A, high half = pair B).
+__device__ __forceinline__ uint32_t row_codes(uint32_t c0, uint32_t c1) { return pack16(0u - c0, 0u - c1); }
+
 // Diagonal candidate of a cell: H(i-1, j-1) minus the mismatch penalty, for both pairs at once.
-// a2 / b2 hold the row / column symbol code of pair A in the low half and of pair B in the high
-// half; min(a ^ b, 1) is 1 per half where they differ (VIMNMX.U16x2, full rate on either pipe),
-// and one IMAD folds the multiplication by the penalty into the subtraction -- it runs on the fma
-// pipe, off the alu pipe that bounds this kernel, and off the row-to-row dependency chain.
-// Works for any number of symbol codes and any penalty (the earlier LOP3 + PRMT table lookup
-// needed codes below 8 and a one-byte penalty).
-__device__ __forceinline__ uint32_t diag_candidate(uint32_t Hd, uint32_t a2, uint32_t b2, uint32_t negD)
+// na2 holds the negated row codes (row_codes()), b2 the column codes, pair A in the low half and
+// pair B in the high half.  The packed add of VIADDMNMX.U16x2 wraps per half, so na + b is zero
+// exactly where the codes agree, and min(na + b, 1) is the 0 / 1 mismatch flag in one alu
+// instruction (min(a ^ b, 1) before: LOP3 + VIMNMX, 2.3 % slower on C3).  One IMAD
+// folds the multiplication by the penalty into the subtraction -- it runs on the fma pipe, off the
+// alu pipe that bounds this kernel, and off the row-to-row dependency chain.  Works for any of the
+// 16 symbol codes and any penalty.
+__device__ __forceinline__ uint32_t diag_candidate(uint32_t Hd, uint32_t na2, uint32_t b2, uint32_t negD)
 {
-    const uint32_t ne = __vminu2(a2 ^ b2, 0x00010001u);
+    const uint32_t ne = __viaddmin_u16x2(na2, b2, 0x00010001u);
     return ne * negD + Hd;
 }
 
@@ -337,7 +344,7 @@ __device__ __forceinline__ void align_two(const AlignArgs& a, long long p0, long
         const int i = itop + r;
         const uint32_t c0 = (i <= A.nA) ? (uint32_t)__ldg(A.xc + min(i, A.nA) - 1) : CODE_PADSYM;
         const uint32_t c1 = (i <= B.nA) ? (uint32_t)__ldg(B.xc + min(i, B.nA) - 1) : CODE_PADSYM;
-        a2[r] = c0 | (c1 << 16);
+        a2[r] = row_codes(c0, c1);
         const uint32_t xb = (uint32_t)f.bias - f.PeoX - (uint32_t)(i - 1) * f.PeeX + 2u;   // Ix(i,0), tagged as state Ix
         Hl[r] = pack16(xb, xb);
         Yn[r] = pack16((uint32_t)f.neg, (uint32_t)f.neg);                                        // no Ix->Iy: Iy(i,1) opens from M only
@@ -470,7 +477,7 @@ __device__ __forceinline__ void align_two_bottom(const AlignArgs& a, long long p
         const int iA = s - offA + 1, iB = s - offB + 1;
         const uint32_t c0 = (iA >= 1) ? (uint32_t)__ldg(A.xc + max(iA, 1) - 1) : CODE_PADSYM;
         const uint32_t c1 = (iB >= 1) ? (uint32_t)__ldg(B.xc + max(iB, 1) - 1) : CODE_PADSYM;
-        a2[r] = c0 | (c1 << 16);
+        a2[r] = row_codes(c0, c1);
         Hl[r] = pack16(col0_H(iA), col0_H(iB));
         // Iy(i, 1): only row 0 has one (the leading end gap, opened from M(0,0)); no Ix->Iy elsewhere
         const uint32_t y0 = (uint32_t)f.bias - f.PeoY + 8u;
@@ -491,81 +498,103 @@ __device__ __forceinline__ void align_two_bottom(const AlignArgs& a, long long p
     uint32_t outX = NEG2, outH = NEG2, finA = 0, finB = 0;
     uint8_t* tbase = trace + (size_t)lane * HB;
     const int tA = A.nB - 1 + (31 - l0), tB = B.nB - 1 + (31 - l0);   // steps at which lane 31 finishes column nB
-    // symbols of y are fetched one step ahead so that the load latency hides behind a whole step
-    // (jj >= -30 always: the pad codes in front of every sequence cover it; past the end the clamp
-    // lands on the pad code behind it)
-    auto fetch_b = [&](int jj, uint32_t& o0, uint32_t& o1) {
-        o0 = (uint32_t)__ldg(A.yc + min(jj, A.nB + 1) - 1);
-        o1 = (uint32_t)__ldg(B.yc + min(jj, B.nB + 1) - 1);
+
+    // Symbols of y travel down the lanes with the wavefront: lane l at step t works on the column
+    // lane l-1 had at step t-1, so one SHFL.UP hands it over.  Lane l0 starts a new column (t + 1)
+    // every step and takes it from a chunk of 32 packed columns that the warp loads together once
+    // every 32 steps, one chunk ahead (lane k: column 32m + k + 1; past the end of a sequence the
+    // clamp lands on the pad code behind it).
+    auto load_chunk = [&](int t0) -> uint32_t {
+        const int jj = t0 + lane + 1;
+        return (uint32_t)__ldg(A.yc + min(jj, A.nB + 1) - 1) | ((uint32_t)__ldg(B.yc + min(jj, B.nB + 1) - 1) << 16);
     };
-    uint32_t nb0, nb1;
-    fetch_b(0 - (lane - l0) + 1, nb0, nb1);
+    uint32_t chunk = 0, next_chunk = load_chunk(0), b2 = 0;
+
+    // One column step.  STEADY: every lane from l0 on is inside the matrix and none is at either
+    // pair's last column, so there is no activity test and no end-column constant.  Lanes below
+    // l0 then compute on garbage (their results are neither stored nor read: lane l0 takes
+    // "minus infinity" from above whatever lane l0 - 1 holds), which costs no issue slot.
     int t = 0;
-#pragma unroll 1
-    for (int seg = 0; seg < 3; ++seg) {   // three segments: see align_two()
-        const int tend = (seg == 0) ? min(tA, tB) + 1 : (seg == 1 ? max(tA, tB) + 1 : nsteps);
-        for (; t < tend; ++t) {
-            const int j = t - (lane - l0) + 1;
-            uint32_t rX = __shfl_up_sync(TAXI_FULL_MASK, outX, 1);
-            uint32_t rH = __shfl_up_sync(TAXI_FULL_MASK, outH, 1);
-            if (lane == 0) { rX = NEG2; rH = NEG2; }   // nothing above slot 0
-            const bool active = live && j >= 1 && j <= nBmax;
-            const uint32_t b0 = nb0, b1 = nb1;
-            fetch_b(j + 1, nb0, nb1);
-            if (active) {
-                const uint32_t b2 = b0 | (b1 << 16);
-                uint32_t ncXM = ncXMi, cXX = cXXi;
-                if (j == A.nB || j == B.nB) {   // a vertical gap in a pair's last column is an end gap
-                    const int xo0 = (j == A.nB) ? f.PeoX : f.PoX, xo1 = (j == B.nB) ? f.PeoX : f.PoX;
-                    const int xe0 = (j == A.nB) ? f.PeeX : f.PeX, xe1 = (j == B.nB) ? f.PeeX : f.PeX;
-                    ncXM = pack16((uint32_t)(1 - xo0), (uint32_t)(1 - xo1));
-                    cXX = 0u - pack16((uint32_t)(xe0 + 2), (uint32_t)(xe1 + 2));
-                }
-                uint32_t Xin = rX;
-                uint32_t tw[WORDS];
-                uint32_t tprev = 0;
-                uint32_t Mr = diag_candidate(Hd_saved, a2[0], b2, f.negD);
-                uint32_t ties = 0, zprev = 0;   // SYM
+    auto step = [&](auto steady) {
+        constexpr bool STEADY = decltype(steady)::value;
+        const uint32_t next_b = __shfl_sync(TAXI_FULL_MASK, chunk, t);   // lane t mod 32: column t + 1
+        b2 = __shfl_up_sync(TAXI_FULL_MASK, b2, 1);
+        uint32_t rX = __shfl_up_sync(TAXI_FULL_MASK, outX, 1);
+        uint32_t rH = __shfl_up_sync(TAXI_FULL_MASK, outH, 1);
+        if (lane == l0) { b2 = next_b; rX = NEG2; rH = NEG2; }   // nothing above slot l0 * H holds a row >= 0
+        const int j = t - (lane - l0) + 1;
+        if (STEADY || (live && j >= 1 && j <= nBmax)) {
+            uint32_t ncXM = ncXMi, cXX = cXXi;
+            if (!STEADY && (j == A.nB || j == B.nB)) {   // a vertical gap in a pair's last column is an end gap
+                const int xo0 = (j == A.nB) ? f.PeoX : f.PoX, xo1 = (j == B.nB) ? f.PeoX : f.PoX;
+                const int xe0 = (j == A.nB) ? f.PeeX : f.PeX, xe1 = (j == B.nB) ? f.PeeX : f.PeX;
+                ncXM = pack16((uint32_t)(1 - xo0), (uint32_t)(1 - xo1));
+                cXX = 0u - pack16((uint32_t)(xe0 + 2), (uint32_t)(xe1 + 2));
+            }
+            uint32_t Xin = rX;
+            uint32_t tw[WORDS];
+            uint32_t tprev = 0;
+            uint32_t Mr = diag_candidate(Hd_saved, a2[0], b2, f.negD);
+            uint32_t ties = 0, zprev = 0;   // SYM
 #pragma unroll
-                for (int r = 0; r < H; ++r) {
-                    uint32_t Mr_next = 0;
-                    if (r + 1 < H) Mr_next = diag_candidate(Hl[r], a2[r + 1], b2, f.negD);   // needs H(i, j-1) before it is overwritten
-                    const uint32_t Yin = Yn[r];
-                    const uint32_t tc = lop3_or3(Mr, Xin, Yin);
-                    const uint32_t Mt = lop3_and_or(Mr, F16_CLEAN, 0x00030003u);
-                    const uint32_t Xt = lop3_and_or(Xin, F16_CLEAN, 0x00020002u);
-                    const uint32_t Yt = lop3_and_or(Yin, F16_CLEAN, 0x00010001u);
-                    Hl[r] = __vimax3_u16x2(Mt, Xt, Yt);
-                    if constexpr (SYM) {
-                        // H ^ Iy ^ 3 is zero per half exactly where H holds Ix's value (tag 2) and Iy the same score
-                        // (tag 1).  min3 over the two rows of a group and 1 gives "no such tie in the group", shifted
-                        // into the lane's bit string on the fma pipe: 2 LOP3 + VIMNMX3 + IMAD per two row pairs.
-                        const uint32_t z = lop3_xor3(Hl[r], Yt, 0x00030003u);
-                        if (r & 1) ties = ties * 2u + __vimin3_u16x2(zprev, z, 0x00010001u);
-                        else if (r == H - 1) ties = ties * 2u + __vminu2(z, 0x00010001u);
-                        zprev = z;
-                    }
-                    Xin = __viaddmax_u16x2(Mt, ncXM, Xt + cXX);
-                    Yn[r] = __viaddmax_u16x2(Mt, (r == H - 1) ? ncYMl : ncYMi, Yt + ((r == H - 1) ? cYYl : cYYi));
-                    if (r & 1) tw[r >> 1] = __byte_perm(tprev, tc, 0x6420);
-                    else if (r == H - 1) tw[r >> 1] = __byte_perm(tc, 0u, 0x6420);
-                    tprev = tc;
-                    Mr = Mr_next;
+            for (int r = 0; r < H; ++r) {
+                uint32_t Mr_next = 0;
+                if (r + 1 < H) Mr_next = diag_candidate(Hl[r], a2[r + 1], b2, f.negD);   // needs H(i, j-1) before it is overwritten
+                const uint32_t Yin = Yn[r];
+                const uint32_t tc = lop3_or3(Mr, Xin, Yin);
+                const uint32_t Mt = lop3_and_or(Mr, F16_CLEAN, 0x00030003u);
+                const uint32_t Xt = lop3_and_or(Xin, F16_CLEAN, 0x00020002u);
+                const uint32_t Yt = lop3_and_or(Yin, F16_CLEAN, 0x00010001u);
+                Hl[r] = __vimax3_u16x2(Mt, Xt, Yt);
+                if constexpr (SYM) {
+                    // H ^ Iy ^ 3 is zero per half exactly where H holds Ix's value (tag 2) and Iy the same score
+                    // (tag 1).  min3 over the two rows of a group and 1 gives "no such tie in the group", shifted
+                    // into the lane's bit string on the fma pipe: 2 LOP3 + VIMNMX3 + IMAD per two row pairs.
+                    const uint32_t z = lop3_xor3(Hl[r], Yt, 0x00030003u);
+                    if (r & 1) ties = ties * 2u + __vimin3_u16x2(zprev, z, 0x00010001u);
+                    else if (r == H - 1) ties = ties * 2u + __vminu2(z, 0x00010001u);
+                    zprev = z;
                 }
-                outX = Xin;
-                outH = Hl[H - 1];
-                Hd_saved = rH;
-                uint4* dst = reinterpret_cast<uint4*>(tbase + (size_t)t * 32 * HB);
-                TAXI_CHECK(a, reinterpret_cast<uint8_t*>(dst) >= trace && reinterpret_cast<uint8_t*>(dst) + HB <= trace + a.trace_per_warp, 4);
+                Xin = __viaddmax_u16x2(Mt, ncXM, Xt + cXX);
+                Yn[r] = __viaddmax_u16x2(Mt, (r == H - 1) ? ncYMl : ncYMi, Yt + ((r == H - 1) ? cYYl : cYYi));
+                if (r & 1) tw[r >> 1] = __byte_perm(tprev, tc, 0x6420);
+                else if (r == H - 1) tw[r >> 1] = __byte_perm(tc, 0u, 0x6420);
+                tprev = tc;
+                Mr = Mr_next;
+            }
+            outX = Xin;
+            outH = Hl[H - 1];
+            Hd_saved = rH;
+            if (STEADY && !live) return;
+            uint4* dst = reinterpret_cast<uint4*>(tbase + (size_t)t * 32 * HB);
+            TAXI_CHECK(a, reinterpret_cast<uint8_t*>(dst) >= trace && reinterpret_cast<uint8_t*>(dst) + HB <= trace + a.trace_per_warp, 4);
 #pragma unroll
-                for (int k = 0; k < HB / 16; ++k) {
-                    uint32_t w[4];
+            for (int k = 0; k < HB / 16; ++k) {
+                uint32_t w[4];
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) w[q] = (4 * k + q < WORDS) ? tw[4 * k + q] : ((SYM && 4 * k + q == WORDS) ? ties : 0u);
-                    __stcg(dst + k, make_uint4(w[0], w[1], w[2], w[3]));
-                }
+                for (int q = 0; q < 4; ++q) w[q] = (4 * k + q < WORDS) ? tw[4 * k + q] : ((SYM && 4 * k + q == WORDS) ? ties : 0u);
+                __stcg(dst + k, make_uint4(w[0], w[1], w[2], w[3]));
             }
         }
+    };
+    auto run = [&](int tend, auto steady) {
+        while (t < tend) {
+            if ((t & 31) == 0) { chunk = next_chunk; next_chunk = load_chunk(t + 32); }
+            const int cend = min(tend, (t | 31) + 1);
+#pragma unroll 1
+            for (; t < cend; ++t) step(steady);
+        }
+    };
+
+    // Five segments: the fill (lanes still starting), the steady state, and three more so that
+    // H(nA, nB) of each pair can be picked up right after the step that produces it (the other
+    // pair may keep the registers busy for more columns) without any capture logic in a loop.
+    const int tfill = 31 - l0;                                   // lane 31 starts column 1
+    const int tsteady = max(tfill, min(A.nB, B.nB) - 1);         // lane l0 reaches the first last column
+#pragma unroll 1
+    for (int seg = 0; seg < 5; ++seg) {
+        if (seg == 1) run(tsteady, std::true_type{});
+        else run(seg == 0 ? tfill : seg == 2 ? min(tA, tB) + 1 : seg == 3 ? max(tA, tB) + 1 : nsteps, std::false_type{});
         if (t - 1 == tA) finA = Hl[H - 1] & 0xFFFFu;
         if (t - 1 == tB) finB = Hl[H - 1] >> 16;
     }
@@ -621,7 +650,7 @@ __device__ __forceinline__ void align_two_bottom_multi(const AlignArgs& a, long 
             const int iA = s - offA + 1, iB = s - offB + 1;
             const uint32_t c0 = (iA >= 1) ? (uint32_t)__ldg(A.xc + max(iA, 1) - 1) : CODE_PADSYM;
             const uint32_t c1 = (iB >= 1) ? (uint32_t)__ldg(B.xc + max(iB, 1) - 1) : CODE_PADSYM;
-            a2[r] = c0 | (c1 << 16);
+        a2[r] = row_codes(c0, c1);
             Hl[r] = pack16(col0_H(iA), col0_H(iB));
             const uint32_t y0 = (uint32_t)f.bias - f.PeoY + 8u;
             Yn[r] = pack16(iA == 0 ? y0 : (uint32_t)f.neg, iB == 0 ? y0 : (uint32_t)f.neg);

@@ -177,6 +177,19 @@ int taxi_best_rows(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t ny
                    int32_t* out_index, double* out_metrics, int32_t* out_counts);
 
 /*
+ * The k closest references of every query row (1 <= k <= 64; anything else is TAXI_E_ARG): the same
+ * blocks as taxi_best_rows, with the k smallest keys (value of metric column `metric`, column index)
+ * of each row selected on the device in ascending order -- smaller value first, equal values by the
+ * smaller column.  NaN is never ranked.  Row x's slots are out_index[x*k .. x*k+k), out_metrics and
+ * out_counts [x*k + r][4] (either may be NULL); a row with fewer than k defined values ends in slots
+ * of index -1, NaN metrics and zero counts.  k = 1 gives taxi_best_rows' results bit for bit.
+ * Column ranges of the same rows from different calls merge on the host: the k smallest keys of
+ * both lists, undefined slots last.
+ */
+int taxi_best_rows_k(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t ny, int32_t metric, int32_t align,
+                     int32_t k, int32_t* out_index, double* out_metrics, int32_t* out_counts);
+
+/*
  * Host-side batch formatter and subset aggregator (no GPU involved; taxi2_b200/csrc/host_format.cpp)
  * for the result files of the tasks: replaces the per-value `str.format` + `.send` writers
  * (distances.py:95-186, 244-279; versus_all.py:278-350) and the per-pair dict aggregation

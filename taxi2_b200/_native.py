@@ -59,6 +59,8 @@ SIGNATURES = {
     "taxi_metrics_from_counts": (C.c_int, [_ctx, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
     "taxi_argmin_rows_device": (C.c_int, [_ctx, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "taxi_best_rows": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "taxi_best_rows_k": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                   C.c_void_p, C.c_void_p, C.c_void_p]),
     "taxi_format_pairs": (C.c_int, [C.c_char_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_double,
                                     C.c_char_p, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]),

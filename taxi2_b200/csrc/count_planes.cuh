@@ -329,4 +329,91 @@ __global__ void best_rows_kernel(const double* __restrict__ metrics, const int32
     }
 }
 
+// The k closest references of every query: per row the k smallest keys (value of metric column
+// `metric`, column index) in ascending order -- for k = 1 the winner of best_rows_kernel.  NaN is
+// never ranked; a row with fewer than k defined values ends in slots of index -1, NaN metrics and
+// zero counts.  Out: [nx][k] indices (offset by col0), [nx][k][4] metrics and counts.
+//
+// One warp per row.  The sorted list lives in registers: lane l holds slots l and 32 + l (the
+// second only when k > 32), empty slots (+inf, BEST_K_NONE), above every real key.  tau is the
+// k-th key.  The warp reads BEST_K_STEPS x 32 columns at a time (loads in flight together), a
+// ballot per 32 picks the lanes whose key is below tau, and each of those few is inserted by the
+// whole warp: a rank from one ballot per slot set, a shift by one lane, tau re-read.  After the
+// first k columns of a barcode row insertions are rare.  The key is a total order, so the list
+// does not depend on the order in which candidates arrive.  No shared memory at any k; 46
+// registers (sm_100a) allow 40 of 64 warps per SM, and capping them at 32 spills.
+constexpr int BEST_K_MAX = 64;
+constexpr int BEST_K_STEPS = 4;
+constexpr int BEST_K_NONE = 0x7fffffff;
+
+__device__ __forceinline__ bool key_less(double v, int c, double tv, int tc) { return v < tv || (v == tv && c < tc); }
+
+__global__ void best_k_rows_kernel(const double* __restrict__ metrics, const int32_t* __restrict__ counts, int32_t nx, int32_t ny,
+                                   int32_t metric, int32_t k, int32_t col0, int32_t* __restrict__ out_idx,
+                                   double* __restrict__ out_metrics, int32_t* __restrict__ out_counts)
+{
+    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= nx) return;
+    const double inf = __longlong_as_double(0x7ff0000000000000LL), nan = __longlong_as_double(0x7ff8000000000000LL);
+    const bool two = k > 32;                  // warp-uniform: the second slot set is in use
+    double v0 = inf, v1 = inf;
+    int c0 = BEST_K_NONE, c1 = BEST_K_NONE;
+    double tv = inf;
+    int tc = BEST_K_NONE;
+    const double* m = metrics + (size_t)row * ny * 4 + metric;
+    for (int base = 0; base < ny; base += 32 * BEST_K_STEPS) {
+        double v[BEST_K_STEPS];
+#pragma unroll
+        for (int u = 0; u < BEST_K_STEPS; ++u) {
+            const int c = base + 32 * u + lane;
+            v[u] = c < ny ? m[(size_t)c * 4] : nan;
+        }
+#pragma unroll
+        for (int u = 0; u < BEST_K_STEPS; ++u) {
+            const int first = base + 32 * u;
+            unsigned cand = __ballot_sync(TAXI_FULL_MASK, v[u] == v[u] && key_less(v[u], first + lane, tv, tc));
+            while (cand) {
+                const int src = __ffs(cand) - 1;
+                cand &= cand - 1;
+                const double cv = __shfl_sync(TAXI_FULL_MASK, v[u], src);
+                const int cc = first + src;
+                if (!key_less(cv, cc, tv, tc)) continue;      // tau has fallen since the ballot
+                int pos = __popc(__ballot_sync(TAXI_FULL_MASK, key_less(v0, c0, cv, cc)));
+                if (two) pos += __popc(__ballot_sync(TAXI_FULL_MASK, key_less(v1, c1, cv, cc)));
+                // slot s takes slot s - 1 above the new key's rank
+                const double u0 = __shfl_up_sync(TAXI_FULL_MASK, v0, 1);
+                const int d0 = __shfl_up_sync(TAXI_FULL_MASK, c0, 1);
+                if (two) {
+                    const double top = __shfl_sync(TAXI_FULL_MASK, v0, 31);
+                    const int ctop = __shfl_sync(TAXI_FULL_MASK, c0, 31);
+                    const double u1 = __shfl_up_sync(TAXI_FULL_MASK, v1, 1);
+                    const int d1 = __shfl_up_sync(TAXI_FULL_MASK, c1, 1);
+                    const int s = 32 + lane;
+                    if (s == pos) { v1 = cv; c1 = cc; }
+                    else if (s > pos) { v1 = lane ? u1 : top; c1 = lane ? d1 : ctop; }
+                }
+                if (lane == pos) { v0 = cv; c0 = cc; }
+                else if (lane > pos) { v0 = u0; c0 = d0; }
+                const int kl = (k - 1) & 31;
+                tv = __shfl_sync(TAXI_FULL_MASK, two ? v1 : v0, kl);
+                tc = __shfl_sync(TAXI_FULL_MASK, two ? c1 : c0, kl);
+            }
+        }
+    }
+    const size_t o = (size_t)row * k;
+    if (lane < k) out_idx[o + lane] = c0 == BEST_K_NONE ? -1 : col0 + c0;
+    if (lane + 32 < k) out_idx[o + 32 + lane] = c1 == BEST_K_NONE ? -1 : col0 + c1;
+    // the winners' four metrics and counts: 8 slots x 4 values per pass, one row's output written contiguously
+    for (int t0 = 0; t0 < 4 * k; t0 += 32) {
+        const int t = t0 + lane, s = t >> 2;
+        const int c = __shfl_sync(TAXI_FULL_MASK, t0 >= 128 ? c1 : c0, s & 31);   // slots of one pass share a set
+        if (t >= 4 * k) continue;
+        const bool none = c == BEST_K_NONE;
+        const size_t at = ((size_t)row * ny + (none ? 0 : c)) * 4 + (t & 3);
+        out_metrics[4 * o + t] = none ? nan : metrics[at];
+        if (counts && out_counts) out_counts[4 * o + t] = none ? 0 : counts[at];
+    }
+}
+
 }  // namespace taxi

@@ -1453,6 +1453,49 @@ int taxi_best_rows(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int32_t ny, 
     return TAXI_OK;
 }
 
+int taxi_best_rows_k(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int32_t ny, int32_t metric, int32_t align,
+                     int32_t k, int32_t* out_index, double* out_metrics, int32_t* out_counts)
+{
+    int rc = check_ctx(c, align != 0);
+    if (rc) return rc;
+    reset_stats(c);
+    if (metric < 0 || metric > 3 || !out_index) return fail(TAXI_E_ARG, "bad argument");
+    if (k < 1 || k > BEST_K_MAX) return fail(TAXI_E_ARG, "k = %d outside 1..%d", k, BEST_K_MAX);
+    if ((rc = check_rect(c, x0, nx, y0, ny))) return rc;
+    if (nx == 0) return TAXI_OK;
+    if (ny == 0) return fail(TAXI_E_ARG, "no columns to reduce over");
+    const long long chunk = align ? kChunkPairs : kCountChunkPairs;
+    if (ny > chunk) return fail(TAXI_E_ARG, "too many columns for one device block (%d > %lld)", ny, chunk);
+    ON_DEVICE(c->device);
+    // a block's selected lists (rows x k slots, k may exceed ny) stay within the block size, like its results (rows x ny pairs)
+    const int32_t rows = (int32_t)std::max<long long>(1, std::min<long long>(nx, chunk / std::max(ny, k)));
+    const uint32_t flags = TAXI_OUT_COUNTS | TAXI_OUT_METRICS;
+    if ((rc = reserve_outputs(c, (long long)rows * ny, flags))) return rc;
+    const size_t kept = (size_t)rows * k;
+    CUDA_TRY(c->d_argidx.reserve(kept));
+    CUDA_TRY(c->d_bestmetrics.reserve(kept * 4));
+    CUDA_TRY(c->d_bestcounts.reserve(kept * 4));
+    for (int32_t r0 = 0; r0 < nx; r0 += rows) {
+        const int32_t nr = std::min(rows, nx - r0);
+        if (align) rc = taxi_align_rect_device(c, x0 + r0, nr, y0, ny, flags, nullptr, c->d_counts.p, c->d_metrics.p);
+        else rc = taxi_count_rect_device(c, x0 + r0, nr, y0, ny, flags, c->d_counts.p, c->d_metrics.p);
+        if (rc) return rc;
+        const int wpb = 8;
+        best_k_rows_kernel<<<(nr + wpb - 1) / wpb, wpb * 32, 0, c->stream>>>(c->d_metrics.p, c->d_counts.p, nr, ny, metric, k, y0,
+                                                                              c->d_argidx.p, c->d_bestmetrics.p, c->d_bestcounts.p);
+        CUDA_TRY(cudaGetLastError());
+        c->launches += 1;
+        const size_t at = (size_t)r0 * k, n = (size_t)nr * k;
+        CUDA_TRY(cudaMemcpyAsync(out_index + at, c->d_argidx.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+        if (out_metrics)
+            CUDA_TRY(cudaMemcpyAsync(out_metrics + 4 * at, c->d_bestmetrics.p, n * 4 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+        if (out_counts)
+            CUDA_TRY(cudaMemcpyAsync(out_counts + 4 * at, c->d_bestcounts.p, n * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+        if ((rc = finish_align(c))) return rc;
+    }
+    return TAXI_OK;
+}
+
 void* taxi_host_alloc(int64_t bytes)
 {
     void* p = nullptr;

@@ -308,6 +308,21 @@ class Engine:
         N.check(self._lib.taxi_best_rows(self._ctx, x0, nx, y0, ny, int(metric), int(bool(align)), _p(index), _p(best), _p(counts)))
         return dict(index=index, metrics=best, counts=counts)
 
+    def best_rows_k(self, x0: int, nx: int, y0: int, ny: int, k: int, metric: int = 0, align: bool = True) -> dict:
+        """The k closest columns of every row x0..x0+nx over [y0, y0+ny), selected on the device
+        (taxi_best_rows_k): per row the k smallest (value of metric column `metric`, column index)
+        in ascending order, NaN never ranked.  index (nx, k) int32, metrics (nx, k, 4) float64,
+        counts (nx, k, 4) int32; slots past a row's defined values hold -1 / NaN / 0.  k = 1 is
+        best_rows with a rank axis."""
+        k = int(k)
+        shape = (nx, max(k, 0))   # the library refuses k outside 1..64
+        index = np.full(shape, -1, dtype=np.int32)
+        best = np.full((*shape, 4), np.nan, dtype=np.float64)
+        counts = np.zeros((*shape, 4), dtype=np.int32)
+        N.check(self._lib.taxi_best_rows_k(self._ctx, x0, nx, y0, ny, int(metric), int(bool(align)), k,
+                                           _p(index), _p(best), _p(counts)))
+        return dict(index=index, metrics=best, counts=counts)
+
     def best_matches(self, metric: int = 0, align: bool = True, rows_per_tile: int | None = None) -> dict:
         """versusReference at scale (BASELINE config C4): best_rows over all of set 0 x all of set 1."""
         return self.best_rows(0, self.n[0], 0, self.ny, metric, align)

@@ -9,8 +9,8 @@ Every pair is independent, so the pair matrix shards with no collective on the d
   (`sharding.assign_tiles`), each GPU's thread walks its share in row order;
 * results are gathered ON THE HOST: every GPU's D2H copy lands directly in its tile's slice of
   one (page-locked) host array, or -- for the best-match row reduction of
-  versus_reference.py:184-188 -- only the per-query winners come back and column tiles of one
-  query are combined on the host with the first-index tie-break.
+  versus_reference.py:184-188 -- only the per-query winners (or k closest references) come back
+  and column tiles of one query are combined on the host with the first-index tie-break.
 
 ctypes releases the GIL for the duration of a native call, so the threads really run concurrently;
 a context is only ever touched by its own thread while a run is in flight.
@@ -371,6 +371,32 @@ class MultiEngine:
             kernel_ms += res["stats"]["kernel_ms"]; cells += res["stats"]["cells"]; launches += res["stats"]["launches"]
         return dict(index=index, metrics=best, counts=counts, kernel_ms=kernel_ms, cells=cells, launches=launches, tiles=len(tiles))
 
+    def best_matches_k(self, k: int, metric: int = 0, align: bool = True, rows_per_tile: int | None = None,
+                       col_tiles: int = 1) -> dict:
+        """The k closest references of every query of set 0 over all of set 1 (Engine.best_rows_k):
+        index (nx, k), metrics and counts (nx, k, 4), ascending by (value of metric column `metric`,
+        reference index).  Tiles are scheduled as in best_matches; with col_tiles > 1 the per-tile
+        lists of a query are merged here (combine_best_k), so the result is the same for any tiling,
+        tile arrival order and number of GPUs."""
+        k = int(k)
+        tiles = self.row_tiles(rows_per_tile, col_tiles)
+        nx = self.nx
+        index = np.full((nx, max(k, 0)), -1, dtype=np.int32)
+        best = np.full((nx, max(k, 0), 4), np.nan, dtype=np.float64)
+        counts = np.zeros((nx, max(k, 0), 4), dtype=np.int32)
+
+        def fn(engine: Engine, tile: Tile, slot: int):
+            res = engine.best_rows_k(tile.x0, tile.nx, tile.y0, tile.ny, k, metric, align)
+            res["stats"] = engine.stats()
+            return res
+
+        kernel_ms = cells = launches = 0
+        for tile, res in self.run_tiles(tiles, fn, depth=4, ordered=False):
+            rows = slice(tile.x0, tile.x0 + tile.nx)
+            combine_best_k(index[rows], best[rows], counts[rows], res["index"], res["metrics"], res["counts"], metric)
+            kernel_ms += res["stats"]["kernel_ms"]; cells += res["stats"]["cells"]; launches += res["stats"]["launches"]
+        return dict(index=index, metrics=best, counts=counts, kernel_ms=kernel_ms, cells=cells, launches=launches, tiles=len(tiles))
+
 
 def _accumulate(acc: dict, engine, redo: bool) -> None:
     st = engine.stats()
@@ -392,3 +418,36 @@ def combine_best(index, best, counts, new_index, new_best, new_counts, metric: i
     index[take] = new_index[take]
     best[take] = new_best[take]
     counts[take] = new_counts[take]
+
+
+def combine_best_k(index, best, counts, new_index, new_best, new_counts, metric: int) -> None:
+    """The k-list counterpart of combine_best: merge another column tile's lists (new_*, (n, k) and
+    (n, k, 4), ascending, undefined slots last as the library returns them) into (index, best,
+    counts) in place.  Each row keeps the k smallest keys (value of metric column `metric`, reference
+    index) of both lists in ascending order; undefined slots (index -1) never displace defined ones and
+    are left as -1 / NaN / 0.  The key is a total order over distinct references, so the result does
+    not depend on the order of the tiles."""
+    k = index.shape[1]
+    if k == 0:
+        return
+    mine, theirs = index[:, 0] >= 0, new_index[:, 0] >= 0
+    # a row with nothing defined yet takes the other list as it is (every row of full-width tiles)
+    take = theirs & ~mine
+    if take.all():
+        index[...], best[...], counts[...] = new_index, new_best, new_counts
+        return
+    index[take] = new_index[take]
+    best[take] = new_best[take]
+    counts[take] = new_counts[take]
+    both = np.flatnonzero(theirs & mine)
+    if not len(both):
+        return
+    idx = np.concatenate([index[both], new_index[both]], axis=1)
+    undefined = idx < 0
+    val = np.where(undefined, np.inf, np.concatenate([best[both, :, metric], new_best[both, :, metric]], axis=1))
+    order = np.lexsort((idx, val, undefined), axis=-1)[:, :k]
+    rows = np.arange(len(both))[:, None]
+    empty = undefined[rows, order]
+    index[both] = np.where(empty, -1, idx[rows, order])
+    best[both] = np.where(empty[..., None], np.nan, np.concatenate([best[both], new_best[both]], axis=1)[rows, order])
+    counts[both] = np.where(empty[..., None], 0, np.concatenate([counts[both], new_counts[both]], axis=1)[rows, order])

@@ -190,6 +190,26 @@ int taxi_best_rows_k(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t 
                      int32_t k, int32_t* out_index, double* out_metrics, int32_t* out_counts);
 
 /*
+ * Every pair within a distance: the same blocks as taxi_best_rows, with the pairs of each block
+ * selected and compacted on the device.  Pair (x, y) is selected iff its value v of metric column
+ * `metric` is not NaN and v * scale <= threshold, one fp64 multiply (scale 100 restates a
+ * percentage threshold exactly as the tasks' `d * 100 <= similarity`); threshold = +inf selects
+ * every defined pair.  A NaN threshold, or a scale that is not finite and positive, is TAXI_E_ARG.
+ * skip_self != 0 drops the pairs (i, i) of set 0 against itself (TAXI_E_ARG with set 1 loaded).
+ * The result is CSR in row-major pair order: out_row_ptr (host int64[nx + 1]) and *out_total, the
+ * number of selected pairs; row x's pairs are entries out_row_ptr[x] .. out_row_ptr[x + 1], in
+ * ascending reference index.  It does not depend on block size or scheduling.  ny = 0 and ny
+ * above one device block are TAXI_E_ARG.
+ * The pairs themselves stay held by the context until the next call that computes on it, and
+ * taxi_pairs_within_fetch copies them out: out_index[total] (column, an index into set 1),
+ * out_metrics[total][4], out_counts[total][4] (either may be NULL).  Fetching with no result held
+ * is TAXI_E_ARG.
+ */
+int taxi_pairs_within(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t ny, int32_t metric, int32_t align,
+                      double threshold, double scale, int32_t skip_self, int64_t* out_row_ptr, int64_t* out_total);
+int taxi_pairs_within_fetch(taxi_ctx* ctx, int32_t* out_index, double* out_metrics, int32_t* out_counts);
+
+/*
  * Host-side batch formatter and subset aggregator (no GPU involved; taxi2_b200/csrc/host_format.cpp)
  * for the result files of the tasks: replaces the per-value `str.format` + `.send` writers
  * (distances.py:95-186, 244-279; versus_all.py:278-350) and the per-pair dict aggregation

@@ -61,6 +61,9 @@ SIGNATURES = {
     "taxi_best_rows": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "taxi_best_rows_k": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                    C.c_void_p, C.c_void_p, C.c_void_p]),
+    "taxi_pairs_within": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double,
+                                    C.c_int32, C.c_void_p, _i64p]),
+    "taxi_pairs_within_fetch": (C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_void_p]),
     "taxi_format_pairs": (C.c_int, [C.c_char_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_double,
                                     C.c_char_p, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]),

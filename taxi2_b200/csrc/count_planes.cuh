@@ -416,4 +416,95 @@ __global__ void best_k_rows_kernel(const double* __restrict__ metrics, const int
     }
 }
 
+// Pairs within a distance (taxi_pairs_within): column c of row r is selected iff its value v of
+// metric column `metric` satisfies v * scale <= threshold -- one fp64 multiply, then the compare, so
+// NaN is never selected -- and, with skip_self, c is not the row's own column r + self0.  Two
+// passes over the block compact the selection into CSR in row-major pair order: within_count_kernel
+// counts per row, an exclusive scan of the counts gives every row its first slot, and
+// within_write_kernel writes each selected pair there.  No atomics: the output is deterministic.
+struct WithinArgs {
+    const double* metrics;   // [nx][ny][4] of the device block
+    const int32_t* counts;   // [nx][ny][4]
+    int32_t nx, ny, metric;
+    double threshold, scale;
+    int32_t self0;           // skip_self: row r's own column is r + self0
+    int32_t skip_self;
+};
+
+constexpr int WITHIN_STEPS = 4;   // 32-column strides of the metric column in flight per warp
+
+__device__ __forceinline__ bool within_pair(const WithinArgs& a, double v, int c, int self)
+{
+    return v * a.scale <= a.threshold && c != self;
+}
+
+// One warp per row, WITHIN_STEPS x 32 columns per iteration (the loads issued together); a ballot
+// per 32 columns, counted with popc.  row_count[r] = selected columns of row r.
+__global__ void within_count_kernel(const WithinArgs a, int32_t* __restrict__ row_count)
+{
+    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= a.nx) return;
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    const double* m = a.metrics + (size_t)row * a.ny * 4 + a.metric;
+    const int self = a.skip_self ? row + a.self0 : -1;
+    int n = 0;
+    for (int base = 0; base < a.ny; base += 32 * WITHIN_STEPS) {
+        double v[WITHIN_STEPS];
+#pragma unroll
+        for (int u = 0; u < WITHIN_STEPS; ++u) {
+            const int c = base + 32 * u + lane;
+            v[u] = c < a.ny ? m[(size_t)c * 4] : nan;
+        }
+#pragma unroll
+        for (int u = 0; u < WITHIN_STEPS; ++u)
+            n += __popc(__ballot_sync(TAXI_FULL_MASK, within_pair(a, v[u], base + 32 * u + lane, self)));
+    }
+    if (lane == 0) row_count[row] = n;
+}
+
+// One warp per row again, same reads.  Row r's pairs go to slots row_off[r] .. row_off[r + 1]: per
+// 32 columns one ballot, and a selected lane's slot is the row's running offset plus the selected
+// lanes below it.  Each selected pair writes its column (offset by col0), its four metrics as one
+// 256-bit store and its four counts as one 128-bit store.  A row stops reading once its last slot
+// is written.
+__global__ void within_write_kernel(const WithinArgs a, const int32_t* __restrict__ row_off, int32_t col0,
+                                    int32_t* __restrict__ out_idx, double* __restrict__ out_metrics,
+                                    int32_t* __restrict__ out_counts)
+{
+    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= a.nx) return;
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    const double* m = a.metrics + (size_t)row * a.ny * 4 + a.metric;
+    const int self = a.skip_self ? row + a.self0 : -1;
+    const unsigned below = (1u << lane) - 1u;
+    int at = row_off[row];
+    const int end = row_off[row + 1];
+    for (int base = 0; base < a.ny && at < end; base += 32 * WITHIN_STEPS) {
+        double v[WITHIN_STEPS];
+#pragma unroll
+        for (int u = 0; u < WITHIN_STEPS; ++u) {
+            const int c = base + 32 * u + lane;
+            v[u] = c < a.ny ? m[(size_t)c * 4] : nan;
+        }
+#pragma unroll
+        for (int u = 0; u < WITHIN_STEPS; ++u) {
+            const int c = base + 32 * u + lane;
+            const bool sel = within_pair(a, v[u], c, self);
+            const unsigned mask = __ballot_sync(TAXI_FULL_MASK, sel);
+            if (sel) {
+                const size_t slot = (size_t)at + __popc(mask & below);
+                const size_t p = (size_t)row * a.ny + c;
+                out_idx[slot] = col0 + c;
+                double r0, r1, r2, r3;
+                asm volatile("ld.global.nc.v4.f64 {%0, %1, %2, %3}, [%4];" : "=d"(r0), "=d"(r1), "=d"(r2), "=d"(r3) : "l"(a.metrics + 4 * p));
+                asm volatile("st.global.L1::no_allocate.L2::evict_first.v4.f64 [%0], {%1, %2, %3, %4};" :: "l"(out_metrics + 4 * slot), "d"(r0), "d"(r1), "d"(r2), "d"(r3) : "memory");
+                __stcs(reinterpret_cast<int4*>(out_counts + 4 * slot), __ldg(reinterpret_cast<const int4*>(a.counts + 4 * p)));
+            }
+            at += __popc(mask);
+        }
+    }
+}
+
 }  // namespace taxi

@@ -4,6 +4,7 @@
 #include "../../include/taxi2_b200.h"
 
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -11,6 +12,8 @@
 #include <mutex>
 #include <string>
 #include <vector>
+
+#include <cub/device/device_scan.cuh>
 
 #include "common.cuh"
 #include "count_planes.cuh"
@@ -58,6 +61,26 @@ template <class T> struct DevBuf {
         return e;
     }
     void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+};
+
+// page-locked host memory, grow-only; growing keeps the first `keep` elements (results gathered over
+// several device blocks), and device-to-host copies into it run at the full link rate
+template <class T> struct HostBuf {
+    T* p = nullptr;
+    size_t cap = 0;  // elements
+    cudaError_t reserve(size_t n, size_t keep)
+    {
+        if (n <= cap) return cudaSuccess;
+        const size_t want = std::max(n, cap + cap / 2);
+        void* q = nullptr;
+        cudaError_t e = cudaHostAlloc(&q, want * sizeof(T), cudaHostAllocPortable);
+        if (e != cudaSuccess) return e;
+        if (keep) std::memcpy(q, p, keep * sizeof(T));
+        if (p) cudaFreeHost(p);
+        p = static_cast<T*>(q); cap = want;
+        return cudaSuccess;
+    }
+    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
 };
 
 // Every entry point runs on its context's device and leaves the calling thread's current device
@@ -141,6 +164,15 @@ struct taxi_ctx {
     DevBuf<unsigned long long> d_redo_count;
     DevBuf<int32_t> d_argidx, d_bestcounts;
     DevBuf<double> d_argval, d_bestmetrics;
+    // taxi_pairs_within: per-row counts and offsets of a block, the scan's scratch, and the held CSR
+    // result (taxi_pairs_within_fetch), dropped by the next call that computes on this context
+    DevBuf<int32_t> d_rowcnt, d_rowoff;
+    DevBuf<uint8_t> d_scantmp;
+    std::vector<int32_t> h_rowoff;
+    HostBuf<int32_t> h_within_idx, h_within_counts;
+    HostBuf<double> h_within_metrics;
+    int64_t within_total = 0;
+    bool within_held = false;
     // stats of the last call
     int64_t launches = 0, cells = 0;
     double kernel_ms = 0.0;
@@ -604,7 +636,8 @@ int download_outputs(taxi_ctx* c, int64_t n, uint32_t flags, int32_t* score, int
     return TAXI_OK;
 }
 
-void reset_stats(taxi_ctx* c) { c->launches = 0; c->cells = 0; c->kernel_ms = 0.0; }
+// at the start of every host-facing compute call; a new computation also drops the held pairs_within result
+void reset_stats(taxi_ctx* c) { c->launches = 0; c->cells = 0; c->kernel_ms = 0.0; c->within_held = false; }
 
 }  // namespace
 
@@ -664,6 +697,8 @@ void taxi_ctx_destroy(taxi_ctx* c)
     c->d_px.release(); c->d_py.release(); c->d_xrows.release(); c->d_ycols.release(); c->d_units.release(); c->d_score.release(); c->d_counts.release(); c->d_metrics.release();
     c->d_alnx.release(); c->d_alny.release(); c->d_alnoff.release(); c->d_alnstart.release();
     c->d_redo.release(); c->d_redo_count.release(); c->d_rscore.release(); c->d_rcounts.release(); c->d_rmetrics.release(); c->d_argidx.release(); c->d_argval.release(); c->d_bestcounts.release(); c->d_bestmetrics.release();
+    c->d_rowcnt.release(); c->d_rowoff.release(); c->d_scantmp.release();
+    c->h_within_idx.release(); c->h_within_counts.release(); c->h_within_metrics.release();
     cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1);
     cudaStreamDestroy(c->stream);
     delete c;
@@ -765,6 +800,7 @@ int taxi_align_rect_device(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int3
 {
     int rc = check_ctx(c, true);
     if (rc) return rc;
+    c->within_held = false;
     if ((rc = check_rect(c, x0, nx, y0, ny))) return rc;
     ON_DEVICE(c->device);
     const long long npairs = (long long)nx * ny;
@@ -946,6 +982,7 @@ int taxi_align_rect_both_device(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0,
 {
     int rc = check_ctx(c, true);
     if (rc) return rc;
+    c->within_held = false;
     if ((rc = check_rect(c, x0, nx, y0, ny))) return rc;
     ON_DEVICE(c->device);
     const long long npairs = (long long)nx * ny;
@@ -1303,6 +1340,7 @@ int taxi_count_rect_device(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int3
 {
     int rc = check_ctx(c, false);
     if (rc) return rc;
+    c->within_held = false;
     if ((rc = check_rect(c, x0, nx, y0, ny))) return rc;
     const long long npairs = (long long)nx * ny;
     if (npairs == 0) return TAXI_OK;
@@ -1382,6 +1420,7 @@ int taxi_metrics_from_counts(taxi_ctx* c, const int32_t* counts, int64_t n, int3
 {
     int rc = check_ctx(c, false);
     if (rc) return rc;
+    c->within_held = false;
     if (n < 0 || (n > 0 && (!counts || !out_metrics)) || (form != 0 && form != 1)) return fail(TAXI_E_ARG, "bad count tuples / form");
     if (n == 0) return TAXI_OK;
     ON_DEVICE(c->device);
@@ -1399,6 +1438,7 @@ int taxi_argmin_rows_device(taxi_ctx* c, const double* d_metrics, int32_t nx, in
 {
     if (!c || !d_metrics || nx < 0 || ny <= 0 || metric < 0 || metric > 3 || !out_index_host)
         return fail(TAXI_E_ARG, "bad argument");
+    c->within_held = false;
     if (nx == 0) return TAXI_OK;
     ON_DEVICE(c->device);
     CUDA_TRY(c->d_argidx.reserve((size_t)nx));
@@ -1493,6 +1533,97 @@ int taxi_best_rows_k(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int32_t ny
             CUDA_TRY(cudaMemcpyAsync(out_counts + 4 * at, c->d_bestcounts.p, n * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
         if ((rc = finish_align(c))) return rc;
     }
+    return TAXI_OK;
+}
+
+int taxi_pairs_within(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int32_t ny, int32_t metric, int32_t align,
+                      double threshold, double scale, int32_t skip_self, int64_t* out_row_ptr, int64_t* out_total)
+{
+    int rc = check_ctx(c, align != 0);
+    if (rc) return rc;
+    reset_stats(c);
+    if (metric < 0 || metric > 3 || !out_row_ptr || !out_total) return fail(TAXI_E_ARG, "bad argument");
+    if (std::isnan(threshold)) return fail(TAXI_E_ARG, "threshold is NaN");
+    if (!std::isfinite(scale) || !(scale > 0.0)) return fail(TAXI_E_ARG, "scale %g is not finite and positive", scale);
+    if (skip_self && c->set[1].loaded) return fail(TAXI_E_ARG, "skip_self needs set 0 as both sets, and set 1 is loaded");
+    if ((rc = check_rect(c, x0, nx, y0, ny))) return rc;
+    out_row_ptr[0] = 0;
+    *out_total = 0;
+    if (nx == 0) {
+        c->within_total = 0;
+        c->within_held = true;
+        return TAXI_OK;
+    }
+    if (ny == 0) return fail(TAXI_E_ARG, "no columns to select from");
+    const long long chunk = align ? kChunkPairs : kCountChunkPairs;
+    if (ny > chunk) return fail(TAXI_E_ARG, "too many columns for one device block (%d > %lld)", ny, chunk);
+    ON_DEVICE(c->device);
+    const int32_t rows = (int32_t)std::max<long long>(1, std::min<long long>(nx, chunk / ny));
+    const uint32_t flags = TAXI_OUT_COUNTS | TAXI_OUT_METRICS;
+    if ((rc = reserve_outputs(c, (long long)rows * ny, flags))) return rc;
+    CUDA_TRY(c->d_rowcnt.reserve((size_t)rows + 1));
+    CUDA_TRY(c->d_rowoff.reserve((size_t)rows + 1));
+    size_t scan_bytes = 0;
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, c->d_rowcnt.p, c->d_rowoff.p, rows + 1, c->stream));
+    CUDA_TRY(c->d_scantmp.reserve(scan_bytes));
+    c->h_rowoff.resize((size_t)rows + 1);
+    WithinArgs a{};
+    a.ny = ny; a.metric = metric; a.threshold = threshold; a.scale = scale; a.skip_self = skip_self != 0;
+    const int wpb = 8;
+    int64_t total = 0;
+    for (int32_t r0 = 0; r0 < nx; r0 += rows) {
+        const int32_t nr = std::min(rows, nx - r0);
+        if (align) rc = taxi_align_rect_device(c, x0 + r0, nr, y0, ny, flags, nullptr, c->d_counts.p, c->d_metrics.p);
+        else rc = taxi_count_rect_device(c, x0 + r0, nr, y0, ny, flags, c->d_counts.p, c->d_metrics.p);
+        if (rc) return rc;
+        a.metrics = c->d_metrics.p; a.counts = c->d_counts.p; a.nx = nr; a.self0 = x0 + r0 - y0;
+        const int grid = (nr + wpb - 1) / wpb;
+        within_count_kernel<<<grid, wpb * 32, 0, c->stream>>>(a, c->d_rowcnt.p);
+        CUDA_TRY(cudaGetLastError());
+        // one count past the last row: the exclusive scan of nr + 1 counts ends in the block total
+        CUDA_TRY(cudaMemsetAsync(c->d_rowcnt.p + nr, 0, sizeof(int32_t), c->stream));
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(c->d_scantmp.p, scan_bytes, c->d_rowcnt.p, c->d_rowoff.p, nr + 1, c->stream));
+        CUDA_TRY(cudaMemcpyAsync(c->h_rowoff.data(), c->d_rowoff.p, ((size_t)nr + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+        c->launches += 2;
+        // also completes the previous block's downloads into the held arrays before they may grow
+        if ((rc = finish_align(c))) return rc;
+        // a block holds at most kCountChunkPairs = 2^27 pairs, so its offsets fit in int32
+        const int32_t n = c->h_rowoff[(size_t)nr];
+        for (int32_t r = 0; r < nr; ++r) out_row_ptr[(size_t)r0 + r + 1] = total + c->h_rowoff[(size_t)r + 1];
+        if (n > 0) {
+            CUDA_TRY(c->d_argidx.reserve((size_t)n, 1));
+            CUDA_TRY(c->d_bestmetrics.reserve((size_t)n * 4, 1));
+            CUDA_TRY(c->d_bestcounts.reserve((size_t)n * 4, 1));
+            const size_t kept = (size_t)total, need = (size_t)total + n;
+            CUDA_TRY(c->h_within_idx.reserve(need, kept));
+            CUDA_TRY(c->h_within_metrics.reserve(need * 4, kept * 4));
+            CUDA_TRY(c->h_within_counts.reserve(need * 4, kept * 4));
+            within_write_kernel<<<grid, wpb * 32, 0, c->stream>>>(a, c->d_rowoff.p, y0, c->d_argidx.p, c->d_bestmetrics.p, c->d_bestcounts.p);
+            CUDA_TRY(cudaGetLastError());
+            c->launches += 1;
+            CUDA_TRY(cudaMemcpyAsync(c->h_within_idx.p + kept, c->d_argidx.p, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+            CUDA_TRY(cudaMemcpyAsync(c->h_within_metrics.p + 4 * kept, c->d_bestmetrics.p, (size_t)n * 4 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+            CUDA_TRY(cudaMemcpyAsync(c->h_within_counts.p + 4 * kept, c->d_bestcounts.p, (size_t)n * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+        }
+        total += n;
+    }
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    c->within_total = total;
+    c->within_held = true;
+    *out_total = total;
+    return TAXI_OK;
+}
+
+int taxi_pairs_within_fetch(taxi_ctx* c, int32_t* out_index, double* out_metrics, int32_t* out_counts)
+{
+    if (!c) return fail(TAXI_E_ARG, "null context");
+    if (!c->within_held) return fail(TAXI_E_ARG, "no taxi_pairs_within result is held (a later call computed on this context, or none ran)");
+    const size_t n = (size_t)c->within_total;
+    if (n == 0) return TAXI_OK;
+    if (!out_index) return fail(TAXI_E_ARG, "null out_index");
+    std::memcpy(out_index, c->h_within_idx.p, n * sizeof(int32_t));
+    if (out_metrics) std::memcpy(out_metrics, c->h_within_metrics.p, n * 4 * sizeof(double));
+    if (out_counts) std::memcpy(out_counts, c->h_within_counts.p, n * 4 * sizeof(int32_t));
     return TAXI_OK;
 }
 

@@ -323,6 +323,25 @@ class Engine:
                                            _p(index), _p(best), _p(counts)))
         return dict(index=index, metrics=best, counts=counts)
 
+    def pairs_within(self, x0: int, nx: int, y0: int, ny: int, threshold: float, metric: int = 0, align: bool = True,
+                     scale: float = 1.0, skip_self: bool = False) -> dict:
+        """Every pair of rows x0..x0+nx x columns [y0, y0+ny) whose value v of metric column `metric`
+        is not NaN and has v * scale <= threshold, selected and compacted on the device
+        (taxi_pairs_within).  CSR in row-major pair order: row_ptr (nx+1,) int64; index (total,)
+        int32, the column (an index into set 1), ascending within a row; metrics (total, 4) float64;
+        counts (total, 4) int32.  scale=100 with a percentage threshold is the tasks' `d * 100 <=
+        similarity`.  skip_self drops the pairs (i, i) of set 0 against itself."""
+        row_ptr = np.zeros(max(nx, 0) + 1, dtype=np.int64)
+        total = C.c_int64(0)
+        N.check(self._lib.taxi_pairs_within(self._ctx, x0, nx, y0, ny, int(metric), int(bool(align)), float(threshold),
+                                            float(scale), int(bool(skip_self)), _p(row_ptr), C.byref(total)))
+        n = total.value
+        index = np.empty(n, dtype=np.int32)
+        metrics = np.empty((n, 4), dtype=np.float64)
+        counts = np.empty((n, 4), dtype=np.int32)
+        N.check(self._lib.taxi_pairs_within_fetch(self._ctx, _p(index), _p(metrics), _p(counts)))
+        return dict(row_ptr=row_ptr, index=index, metrics=metrics, counts=counts)
+
     def best_matches(self, metric: int = 0, align: bool = True, rows_per_tile: int | None = None) -> dict:
         """versusReference at scale (BASELINE config C4): best_rows over all of set 0 x all of set 1."""
         return self.best_rows(0, self.n[0], 0, self.ny, metric, align)

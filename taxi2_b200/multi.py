@@ -10,7 +10,8 @@ Every pair is independent, so the pair matrix shards with no collective on the d
 * results are gathered ON THE HOST: every GPU's D2H copy lands directly in its tile's slice of
   one (page-locked) host array, or -- for the best-match row reduction of
   versus_reference.py:184-188 -- only the per-query winners (or k closest references) come back
-  and column tiles of one query are combined on the host with the first-index tie-break.
+  and column tiles of one query are combined on the host with the first-index tie-break; the
+  pairs within a threshold come back as per-tile CSR pieces, assembled on the host.
 
 ctypes releases the GIL for the duration of a native call, so the threads really run concurrently;
 a context is only ever touched by its own thread while a run is in flight.
@@ -397,6 +398,30 @@ class MultiEngine:
             kernel_ms += res["stats"]["kernel_ms"]; cells += res["stats"]["cells"]; launches += res["stats"]["launches"]
         return dict(index=index, metrics=best, counts=counts, kernel_ms=kernel_ms, cells=cells, launches=launches, tiles=len(tiles))
 
+    def pairs_within(self, threshold: float, metric: int = 0, align: bool = True, scale: float = 1.0, skip_self: bool = False,
+                     rows_per_tile: int | None = None, col_tiles: int = 1) -> dict:
+        """Every pair of set 0 x set 1 (or set 0 x set 0) whose value of metric column `metric`,
+        times `scale`, is at most `threshold` (Engine.pairs_within): one CSR over all of set 0,
+        row_ptr (nx+1,), index (total,), metrics and counts (total, 4), row-major with ascending
+        reference index within a row.  Tiles are scheduled as in best_matches; the per-tile pieces
+        are assembled here (combine_within), so the result is the same for any tiling, tile
+        arrival order and number of GPUs."""
+        tiles = self.row_tiles(rows_per_tile, col_tiles)
+
+        def fn(engine: Engine, tile: Tile, slot: int):
+            res = engine.pairs_within(tile.x0, tile.nx, tile.y0, tile.ny, threshold, metric, align, scale, skip_self)
+            res["stats"] = engine.stats()
+            return res
+
+        pieces = []
+        kernel_ms = cells = launches = 0
+        for tile, res in self.run_tiles(tiles, fn, depth=4, ordered=False):
+            pieces.append((tile.x0, tile.nx, tile.y0, res))
+            kernel_ms += res["stats"]["kernel_ms"]; cells += res["stats"]["cells"]; launches += res["stats"]["launches"]
+        out = combine_within(pieces, self.nx)
+        out.update(kernel_ms=kernel_ms, cells=cells, launches=launches, tiles=len(tiles))
+        return out
+
 
 def _accumulate(acc: dict, engine, redo: bool) -> None:
     st = engine.stats()
@@ -451,3 +476,34 @@ def combine_best_k(index, best, counts, new_index, new_best, new_counts, metric:
     index[both] = np.where(empty, -1, idx[rows, order])
     best[both] = np.where(empty[..., None], np.nan, np.concatenate([best[both], new_best[both]], axis=1)[rows, order])
     counts[both] = np.where(empty[..., None], 0, np.concatenate([counts[both], new_counts[both]], axis=1)[rows, order])
+
+
+def combine_within(tiles, nx: int) -> dict:
+    """Assemble the CSR pieces of taxi_pairs_within calls over tiles of rows 0..nx into one CSR.
+    `tiles` holds (x0, nx, y0, piece), piece = dict(row_ptr, index, metrics, counts) of rows x0..x0+nx
+    over columns from y0 on, in any order.  A row's segments are placed in ascending y0 (the column
+    ranges of one row's tiles are disjoint), so every row lists its pairs in ascending reference
+    index and the result is the same for any tiling and arrival order.  Per tile a few numpy
+    operations: a tile that holds whole rows is one slice copy, otherwise one scatter."""
+    tiles = sorted(tiles, key=lambda t: (t[2], t[0]))
+    per_row = np.zeros(nx, dtype=np.int64)
+    for x0, n, _, piece in tiles:
+        per_row[x0:x0 + n] += np.diff(piece["row_ptr"])
+    row_ptr = np.zeros(nx + 1, dtype=np.int64)
+    np.cumsum(per_row, out=row_ptr[1:])
+    total = int(row_ptr[-1])
+    index = np.empty(total, dtype=np.int32)
+    metrics = np.empty((total, 4), dtype=np.float64)
+    counts = np.empty((total, 4), dtype=np.int32)
+    fill = row_ptr[:-1].copy()   # the next free entry of every row
+    for x0, n, _, piece in tiles:
+        lens = np.diff(piece["row_ptr"])
+        if np.array_equal(lens, per_row[x0:x0 + n]):   # the tile holds all of its rows' pairs
+            dst = slice(int(row_ptr[x0]), int(row_ptr[x0 + n]))
+        else:
+            dst = np.repeat(fill[x0:x0 + n] - piece["row_ptr"][:-1], lens) + np.arange(int(piece["row_ptr"][-1]))
+        index[dst] = piece["index"]
+        metrics[dst] = piece["metrics"]
+        counts[dst] = piece["counts"]
+        fill[x0:x0 + n] += lens
+    return dict(row_ptr=row_ptr, index=index, metrics=metrics, counts=counts)

@@ -643,7 +643,7 @@ def test_tensor_core_counts_equal_popcount_and_oracle(engine, case):
 
 
 def test_table_form_of_the_metric_epilogue(engine):
-    """Rows of at most 2048 columns take JC / K2P from a fixed-point table of ln k (exact integer
+    """Rows of at most 1920 columns take JC / K2P from a fixed-point table of ln k (exact integer
     differences) instead of the floating-point formula.  Every (n, ts, tv) combination short rows
     can produce -- including the ones whose logarithm argument is exactly zero, where the
     reference's rounding decides between None and a finite value -- against the oracle and against

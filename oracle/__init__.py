@@ -12,5 +12,6 @@ from .oracle import (  # noqa: F401
     count_pairs,
     max_threads,
     metrics,
+    metrics_batch,
     uses_gotoh,
 )

@@ -42,6 +42,8 @@ def _load():
         lib.taxi_oracle_count.restype = C.c_int
         lib.taxi_oracle_metrics.argtypes = [i32p, f64p]
         lib.taxi_oracle_metrics.restype = None
+        lib.taxi_oracle_metrics_batch.argtypes = [i32p, C.c_int64, f64p]
+        lib.taxi_oracle_metrics_batch.restype = None
         lib.taxi_oracle_uses_gotoh.argtypes = [f64p]
         lib.taxi_oracle_uses_gotoh.restype = C.c_int
         lib.taxi_oracle_max_threads.restype = C.c_int
@@ -100,6 +102,15 @@ def metrics(counts) -> tuple[float, float, float, float]:
     out = (C.c_double * 4)()
     _load().taxi_oracle_metrics(cin, out)
     return tuple(out)
+
+
+def metrics_batch(counts) -> np.ndarray:
+    """(n, 4) count tuples -> (n, 4) float64 {p, p-gaps, jc, k2p}: `metrics` of each tuple in one call."""
+    counts = np.ascontiguousarray(counts, dtype=np.int32).reshape(-1, 4)
+    out = np.empty((len(counts), 4), np.float64)
+    _load().taxi_oracle_metrics_batch(counts.ctypes.data_as(C.POINTER(C.c_int32)), len(counts),
+                                      out.ctypes.data_as(C.POINTER(C.c_double)))
+    return out
 
 
 def align_count_pairs(seqs: np.ndarray, offsets: np.ndarray, px: np.ndarray, py: np.ndarray,

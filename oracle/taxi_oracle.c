@@ -285,6 +285,12 @@ void taxi_oracle_metrics(const int32_t counts[4], double out[4])
     out[3] = isfinite(k2p) ? k2p + 0.0 : NAN;
 }
 
+/* taxi_oracle_metrics of n count tuples (counts int32[n][4] -> out double[n][4]) */
+void taxi_oracle_metrics_batch(const int32_t* counts, int64_t n, double* out)
+{
+    for (int64_t k = 0; k < n; ++k) taxi_oracle_metrics(counts + 4 * k, out + 4 * k);
+}
+
 /*
  * The whole per-pair path of versus_all.py:527-552 for a list of pairs:
  * align (Biopython restatement) -> 4 counts -> 4 metrics.  Used as the CPU baseline

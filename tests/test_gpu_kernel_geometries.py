@@ -7,6 +7,9 @@ that select it (row counts up to GENERAL_LIMIT / PACKED_LIMIT), with y lengths o
 full window.  Each launch is compared with the oracle -- scores and counts bit for bit, p / p-gaps
 bit for bit, JC / K2P within 1e-12, gapped strings for a bounded subset -- and `last_kernel` with
 the instance the restatement predicts, so that no case passes on another instance by accident.
+The metrics every instance writes are also bit for bit `taxi_metrics_from_counts` of its own counts
+(floating-point form, NaN pattern included): each instance inlines its own copy of the epilogue, and
+the entry point is the copy test_gpu_metric_arithmetic.py pins against exact references.
 
 The both-orientations kernel (`gotoh_pair16_kernel<H,1,true>`) keeps its tie bits in a word whose
 layout depends on H; a missed bit writes a wrong (y, x) result.  Each of its six geometries gets a
@@ -209,6 +212,17 @@ def assert_same(got: dict, want: dict, where):
     assert_metrics_close(got["metrics"].reshape(-1, 4), want["metrics"].reshape(-1, 4))
 
 
+def assert_epilogue(engine, got: dict, where):
+    """The metrics a kernel wrote are bit for bit the floating-point form of taxi_metrics_from_counts
+    of the counts it wrote: one contraction or rounding step that differs between the two copies of
+    the epilogue moves a value by an ulp, and pairs_within / best-k decide on exact values."""
+    counts = got["counts"].reshape(-1, 4)
+    want = engine.metrics_from_counts(counts, table=False)
+    bits = got["metrics"].reshape(-1, 4).view(np.uint64)
+    bad = np.flatnonzero((bits != want.view(np.uint64)).any(axis=1))
+    assert len(bad) == 0, (where, counts[bad][:4].tolist(), got["metrics"].reshape(-1, 4)[bad][:4].tolist(), want[bad][:4].tolist())
+
+
 def run_pairs(engine, xs, ys, scores, opts, family, H, strings=True):
     """Pair list against the oracle; the predicted instance must be (family, H) and must have run."""
     la, lb = [len(x) for x in xs], [len(y) for y in ys]
@@ -226,14 +240,19 @@ def run_pairs(engine, xs, ys, scores, opts, family, H, strings=True):
         where = (K.name(family, H), scores, predicted, kernel)
         assert kernel == K.CODE[family], where
         assert_same(got, want, where)
+        assert_epilogue(engine, got, where)
         if strings:
             sub = [k for k in range(n) if la[k] * lb[k] <= STRING_CELLS]
             sub_pred = K.instance(scores, [la[k] for k in sub], [lb[k] for k in sub], "pairs", opts)
-            ax, ay, sc = engine.align_strings(px[sub], px[sub])
+            ox, oy, start, off, sc, res = engine.align_strings_raw(px[sub], px[sub], want=("counts", "metrics"))
             assert engine.last_kernel == K.CODE[sub_pred[0]], (where, sub_pred)
             assert np.array_equal(sc, want["score"][sub]), where
+            assert np.array_equal(res["counts"], want["counts"][sub]), where
+            assert_epilogue(engine, res, (where, "strings"))
+            bx, by = ox.tobytes(), oy.tobytes()
             for i, k in enumerate(sub):
-                assert (ax[i].decode("latin-1"), ay[i].decode("latin-1")) == oracle.align(xs[k], ys[k], scores)[:2], (where, k)
+                ax, ay = bx[int(start[i]):int(off[i + 1])], by[int(start[i]):int(off[i + 1])]
+                assert (ax.decode("latin-1"), ay.decode("latin-1")) == oracle.align(xs[k], ys[k], scores)[:2], (where, k)
     return got, predicted
 
 
@@ -284,6 +303,8 @@ def check_both(engine, xs, ys, H, tie_rich):
     want_yx = want_xy if ys is xs else oracle_batch(ys, xs, qy, qx, DEFAULT)
     assert_same(xy, want_xy, (H, "xy"))
     assert_same(yx, want_yx, (H, "yx"))
+    assert_epilogue(engine, xy, (H, "xy"))
+    assert_epilogue(engine, yx, (H, "yx"))      # mirrored from the (x, y) pass or re-aligned
     c_xy = want_xy["counts"].reshape(nx, ny, 4)
     c_yx = want_yx["counts"].reshape(ny, nx, 4)
     asymmetric = int((c_xy != np.swapaxes(c_yx, 0, 1)).any(axis=2).sum())

@@ -246,11 +246,26 @@ int taxi_format_matrix(const char* path, const char* xid_bytes, const int64_t* x
     return format_rows(path, nx, threads, fn);
 }
 
+// A gapped string holds one latin-1 byte per symbol (the sequences went in as str.encode("latin-1"));
+// the file holds the UTF-8 text of that str, as the Python handler writes it: bytes 0x80-0xFF take two.
+static void append_latin1_as_utf8(std::string& out, const uint8_t* s, size_t len)
+{
+    for (size_t k = 0; k < len; ++k) {
+        const uint8_t c = s[k];
+        if (c < 0x80) {
+            out += (char)c;
+        } else {
+            out += (char)(0xC0 | (c >> 6));
+            out += (char)(0x80 | (c & 0x3F));
+        }
+    }
+}
+
 // SequencePairHandler.Formatted records (pairs.py:51-97) for the nx*ny pairs of a row block, pair
 // p = (x0 + p / ny, p % ny): "idx / idy", aligned x, the match pattern ('|' equal and not a gap, '-'
-// either is a gap, '.' otherwise), aligned y; records are separated by one empty line, so every
-// record but the file's first is preceded by "\n".  The gapped strings are the right-aligned
-// slots taxi_align_strings fills: pair p occupies [aln_start[p], aln_off[p + 1]).
+// either is a gap, '.' otherwise; one character per symbol), aligned y; records are separated by one
+// empty line, so every record but the file's first is preceded by "\n".  The gapped strings are the
+// right-aligned slots taxi_align_strings fills: pair p occupies [aln_start[p], aln_off[p + 1]).
 int taxi_format_aligned_pairs(const char* path, int32_t first_record,
                               const char* xid_bytes, const int64_t* xid_off, const char* yid_bytes, const int64_t* yid_off,
                               int32_t x0, int32_t nx, int32_t ny,
@@ -275,7 +290,11 @@ int taxi_format_aligned_pairs(const char* path, int32_t first_record,
                 const uint8_t* ax = aln_x + aln_start[p];
                 const uint8_t* ay = aln_y + aln_start[p];
                 const size_t len = (size_t)(aln_off[p + 1] - aln_start[p]);
-                out.append(reinterpret_cast<const char*>(ax), len);
+                uint8_t high = 0;   // any byte >= 0x80 in either string: the UTF-8 path
+                for (size_t k = 0; k < len; ++k) high |= ax[k] | ay[k];
+                const bool ascii = high < 0x80;
+                if (ascii) out.append(reinterpret_cast<const char*>(ax), len);
+                else append_latin1_as_utf8(out, ax, len);
                 out += '\n';
                 const size_t at = out.size();
                 out.resize(at + len);
@@ -289,7 +308,8 @@ int taxi_format_aligned_pairs(const char* path, int32_t first_record,
                     pat[k] = (char)(('-' & gap) | (base & (uint8_t)~gap));
                 }
                 out += '\n';
-                out.append(reinterpret_cast<const char*>(ay), len);
+                if (ascii) out.append(reinterpret_cast<const char*>(ay), len);
+                else append_latin1_as_utf8(out, ay, len);
                 out += '\n';
             }
         }

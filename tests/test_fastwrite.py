@@ -174,6 +174,41 @@ def test_aligned_pair_records_match_the_python_handler(tmp_path):
     assert out.read_bytes() == (Path(__file__).parent / "golden" / "pairs_simple.formatted").read_bytes()
 
 
+def test_aligned_pair_records_on_every_byte_value(tmp_path):
+    """Gapped strings over every byte 0x01-0xFF (ASCII ids): the library writes the UTF-8 text of
+    the latin-1 symbols, byte for byte what SequencePairHandler.Formatted writes for the decoded str
+    (0xC9 'É' -> C3 89), with one pattern character per symbol; ASCII records stay as they are."""
+    from taxi2_b200.pairs import SequencePair, SequencePairHandler
+
+    rng = np.random.default_rng(255)
+    every = np.arange(1, 256, dtype=np.uint8)
+    pairs = [(every.tobytes(), every.tobytes()), (every.tobytes(), every[::-1].tobytes()),
+             (b"AC\xc9GT-", b"AC\xc9G-T"), (b"ACGT", b"AC-T")]
+    for _ in range(6):
+        n = int(rng.integers(1, 300))
+        pairs.append((every[rng.integers(0, 255, n)].tobytes(), every[rng.integers(0, 255, n)].tobytes()))
+    ny = 2
+    nx = len(pairs) // ny
+    slots = [len(ax) + int(rng.integers(0, 5)) for ax, _ in pairs]
+    off = np.concatenate([[0], np.cumsum(slots)]).astype(np.int64)
+    start = np.array([off[k + 1] - len(pairs[k][0]) for k in range(len(pairs))], dtype=np.int64)
+    ox = np.zeros(int(off[-1]), dtype=np.uint8)
+    oy = np.zeros(int(off[-1]), dtype=np.uint8)
+    for k, (ax, ay) in enumerate(pairs):
+        ox[start[k]:off[k + 1]] = np.frombuffer(ax, dtype=np.uint8)
+        oy[start[k]:off[k + 1]] = np.frombuffer(ay, dtype=np.uint8)
+    xids, yids = [f"x{i}" for i in range(nx)], [f"y{j}" for j in range(ny)]
+    want = tmp_path / "want.txt"
+    with SequencePairHandler.Formatted(want, "w") as file:
+        for k, (ax, ay) in enumerate(pairs):
+            file.write(SequencePair(Sequence(xids[k // ny], ax.decode("latin-1")), Sequence(yids[k % ny], ay.decode("latin-1"))))
+    got = tmp_path / "got.txt"
+    got.write_bytes(b"")
+    fw.format_aligned_pairs(got, True, fw.StringTable(xids), fw.StringTable(yids), 0, nx, ny, ox, oy, start, off, threads=2)
+    assert got.read_bytes() == want.read_bytes()
+    assert b"\nx1 / y0\nAC\xc3\x89GT-\n||||--\nAC\xc3\x89G-T\n\nx1 / y1\nACGT\n||-|\nAC-T\n" in got.read_bytes()
+
+
 @pytest.mark.parametrize("spec", ["{:.4f}", "{:.0f}", "{:.2f}", "{:.9f}", "{:f}"])
 def test_fixed_point_fast_path_equals_python_format(tmp_path, spec):
     """The integer-arithmetic formatter behind "%.Nf" (host_format.cpp: append_fixed) against

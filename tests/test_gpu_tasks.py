@@ -132,6 +132,44 @@ def test_versus_reference_outputs(tmp_path, align, multiply, main, native):
     assert_same_tree(task.work_dir, tmp_path / "want")
 
 
+def with_accented_letters(records):
+    """A few sequences carrying letters outside ASCII ('É', 'ü'), as a UTF-8 input file can hold."""
+    out = list(records)
+    for k, (at, letters) in enumerate(((5, "É"), (40, "üü"), (90, "ÉüÉ"))):
+        s = out[k]
+        out[k] = Sequence(s.id, s.seq[:at] + letters + s.seq[at:], s.extras)
+    return out
+
+
+@pytest.mark.parametrize("native", [True, False])
+def test_aligned_pairs_with_letters_outside_ascii(tmp_path, native):
+    """VersusAll and VersusReference with aligned pairs on sequences with 'É' / 'ü': the native and
+    the Python writers and the restated reference pipeline write the same bytes -- the UTF-8 text of
+    the aligned strings."""
+    seqs, species, genera = load("Taxi2test1_10.tab")
+    records = with_accented_letters(seqs)
+    task = VersusAll()
+    task.work_dir = tmp_path / "got"
+    task.progress_handler = SILENT
+    task.input.sequences = Sequences(records)
+    task.input.species, task.input.genera = species, genera
+    task.native_writers = native
+    task.start()
+    ref_pipeline.versus_all(records, tmp_path / "want", species, genera)
+    assert "É".encode("utf-8") in (task.work_dir / "align" / "aligned_pairs.txt").read_bytes()
+    assert_same_tree(task.work_dir, tmp_path / "want")
+
+    data, reference = records[:4], records[3:]
+    task = VersusReference()
+    task.work_dir = tmp_path / "got_ref"
+    task.progress_handler = SILENT
+    task.input.data, task.input.reference = Sequences(data), Sequences(reference)
+    task.native_writers = native
+    task.start()
+    ref_pipeline.versus_reference(data, reference, tmp_path / "want_ref", align=True, metric=DistanceMetric.fromLabel("p"))
+    assert_same_tree(task.work_dir, tmp_path / "want_ref")
+
+
 def test_versus_reference_raises_without_any_defined_distance(tmp_path):
     task = VersusReference()
     task.work_dir = tmp_path / "got"

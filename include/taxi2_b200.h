@@ -210,6 +210,32 @@ int taxi_pairs_within(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t
 int taxi_pairs_within_fetch(taxi_ctx* ctx, int32_t* out_index, double* out_metrics, int32_t* out_counts);
 
 /*
+ * Clusters within a distance: single-linkage components of set 0 (operational taxonomic units at
+ * a distance threshold), linked and united on the device.  The nodes are the n sequences of set 0,
+ * which serves as both sets (TAXI_E_ARG with set 1 loaded).  The call computes the rectangle rows
+ * [x0, x0+nx) x columns [y0, y0+ny) of set 0 x set 0 in the blocks of taxi_pairs_within and links
+ * x and y at threshold t iff the pair (x, y) has a value v of metric column `metric` that is not
+ * NaN and v * scale <= thresholds[t] -- taxi_pairs_within's predicate; the pairs (i, i) link
+ * nothing.  Links are undirected: over the full square, x and y are linked if either orientation
+ * qualifies.  Every threshold (1 .. TAXI_CLUSTER_MAX_THRESHOLDS of them, in any order) is evaluated
+ * on its own, bit for bit as one call per threshold.
+ * out_label (host int32[nthresholds][n]): out_label[t][i] is the smallest set-0 index in i's
+ * connected component at threshold t, so a node without links labels itself.  The labels do not
+ * depend on block size, scheduling, tiling or the number of devices.
+ * seed (host int32[nthresholds][n], or NULL for singletons) starts every component from an earlier
+ * labeling, so that calls compose: two calls over disjoint row ranges, the second seeded with the
+ * first's out_label (seed may be out_label itself), equal one call over both.  Each row of the seed
+ * must be canonical: seed[t][i] <= i and seed[t][seed[t][i]] == seed[t][i].
+ * TAXI_E_ARG: nthresholds outside 1 .. TAXI_CLUSTER_MAX_THRESHOLDS, a NaN threshold, a scale that is
+ * not finite and positive, a metric outside 0 .. 3, null thresholds or out_label, a seed that is not
+ * canonical, ny = 0 or above one device block (nx = 0 included).  A refused call leaves out_label
+ * untouched.  nx = 0 with valid arguments returns the seed (or the singletons).
+ */
+#define TAXI_CLUSTER_MAX_THRESHOLDS 8
+int taxi_clusters_within(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t ny, int32_t metric, int32_t align,
+                         const double* thresholds, int32_t nthresholds, double scale, const int32_t* seed, int32_t* out_label);
+
+/*
  * Host-side batch formatter and subset aggregator (no GPU involved; taxi2_b200/csrc/host_format.cpp)
  * for the result files of the tasks: replaces the per-value `str.format` + `.send` writers
  * (distances.py:95-186, 244-279; versus_all.py:278-350) and the per-pair dict aggregation

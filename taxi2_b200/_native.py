@@ -64,6 +64,8 @@ SIGNATURES = {
     "taxi_pairs_within": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double,
                                     C.c_int32, C.c_void_p, _i64p]),
     "taxi_pairs_within_fetch": (C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "taxi_clusters_within": (C.c_int, [_ctx, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
+                                       C.c_double, C.c_void_p, C.c_void_p]),
     "taxi_format_pairs": (C.c_int, [C.c_char_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_double,
                                     C.c_char_p, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]),

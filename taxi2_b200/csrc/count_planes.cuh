@@ -28,6 +28,8 @@
 // scan that starts at the first word where both sequences have real columns (normally it looks
 // at one word per end).
 #pragma once
+#include <cuda/atomic>
+
 #include "common.cuh"
 
 namespace taxi {
@@ -504,6 +506,113 @@ __global__ void within_write_kernel(const WithinArgs a, const int32_t* __restric
             }
             at += __popc(mask);
         }
+    }
+}
+
+// Clusters within a distance (taxi_clusters_within): single-linkage components of set 0 at up to
+// CLUSTER_MAX_THRESHOLDS thresholds in one pass, one union-find forest of the n nodes per threshold,
+// lock-free in the style of ECL-CC (Jaiganesh and Burtscher, HPDC 2018).  parent[x] <= x always
+// holds; a hook CASes the LARGER root's parent from itself to the smaller root, so the root of every
+// component is its minimum and the labels are canonical without a relabelling pass.  find halves the
+// path with relaxed loads and stores: a parent only ever moves to an ancestor inside its component,
+// so a stale load or an overwritten halving leaves a valid forest, at worst a longer path.
+constexpr int CLUSTER_MAX_THRESHOLDS = 8;
+static_assert(CLUSTER_MAX_THRESHOLDS * WITHIN_STEPS <= 32, "one selection bit per (step, threshold) in a 32-bit word");
+
+struct LinkArgs {
+    const double* metrics;   // [nx][ny][4] of the device block
+    int32_t nx, ny, metric;
+    double scale;
+    double threshold[CLUSTER_MAX_THRESHOLDS];
+    uint32_t live;           // bit CLUSTER_MAX_THRESHOLDS * u + t set for every step u and threshold t < nt
+    int32_t x0, y0;          // set-0 index of the block's row 0 and column 0
+    int32_t n;               // nodes of one forest
+    int32_t* parent;         // [nt][n]
+};
+
+using uf_ref = cuda::atomic_ref<int32_t, cuda::thread_scope_device>;
+
+__device__ __forceinline__ int32_t uf_load(int32_t* parent, int32_t x)
+{
+    return uf_ref(parent[x]).load(cuda::memory_order_relaxed);
+}
+
+__device__ __forceinline__ int32_t uf_find(int32_t* parent, int32_t x)
+{
+    int32_t cur = uf_load(parent, x);
+    if (cur == x) return x;
+    int32_t prev = x, next;
+    while (cur > (next = uf_load(parent, cur))) {
+        uf_ref(parent[prev]).store(next, cuda::memory_order_relaxed);
+        prev = cur;
+        cur = next;
+    }
+    return cur;
+}
+
+__device__ __forceinline__ void uf_unite(int32_t* parent, int32_t a, int32_t b)
+{
+    a = uf_find(parent, a);
+    b = uf_find(parent, b);
+    while (a != b) {
+        if (a > b) { const int32_t t = a; a = b; b = t; }
+        const int32_t seen = atomicCAS(parent + b, b, a);   // relaxed
+        if (seen == b) return;
+        b = uf_find(parent, seen);   // b was hooked under another root meanwhile: go on from there
+    }
+}
+
+// One warp per row, the metric column read as within_count_kernel reads it.  Per WITHIN_STEPS x 32
+// columns every lane gathers one bit per (step, threshold) -- v * scale <= threshold, the predicate
+// of within_pair, never true for NaN or the pair (x, x) -- and a warp-wide OR skips the columns that
+// link nothing.  A set bit unites (x0 + row, y0 + column) in that threshold's forest.
+__global__ void link_within_kernel(const LinkArgs a)
+{
+    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= a.nx) return;
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    const double* m = a.metrics + (size_t)row * a.ny * 4 + a.metric;
+    const int32_t x = a.x0 + row;
+    const int self = x - a.y0;   // the column of the pair (x, x)
+    for (int base = 0; base < a.ny; base += 32 * WITHIN_STEPS) {
+        double v[WITHIN_STEPS];
+#pragma unroll
+        for (int u = 0; u < WITHIN_STEPS; ++u) {
+            const int c = base + 32 * u + lane;
+            v[u] = c < a.ny ? m[(size_t)c * 4] : nan;
+        }
+        uint32_t sel = 0;
+#pragma unroll
+        for (int u = 0; u < WITHIN_STEPS; ++u) {
+            const double s = v[u] * a.scale;
+            const bool other = base + 32 * u + lane != self;
+#pragma unroll
+            for (int t = 0; t < CLUSTER_MAX_THRESHOLDS; ++t)
+                sel |= (uint32_t)(other && s <= a.threshold[t]) << (CLUSTER_MAX_THRESHOLDS * u + t);
+        }
+        sel &= a.live;
+        for (uint32_t any = __reduce_or_sync(TAXI_FULL_MASK, sel); any; any &= any - 1) {
+            const int bit = __ffs(any) - 1;
+            if (sel >> bit & 1u) {
+                const int u = bit / CLUSTER_MAX_THRESHOLDS, t = bit % CLUSTER_MAX_THRESHOLDS;
+                uf_unite(a.parent + (size_t)t * a.n, x, a.y0 + base + 32 * u + lane);
+            }
+        }
+    }
+}
+
+// label = root, in place, one thread per (node, forest) and blockIdx.y the forest.  It runs after
+// every link of the call, so no root changes any more; the walk only loads (no halving), so every
+// parent a thread reads is an ancestor of its node and the stores of other threads -- each the root
+// of its own node -- cannot send it elsewhere.
+__global__ void flatten_kernel(int32_t* parent, int32_t n)
+{
+    int32_t* p = parent + (size_t)blockIdx.y * n;
+    for (int32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        int32_t r = uf_load(p, i), next;
+        while (r != (next = uf_load(p, r))) r = next;
+        uf_ref(p[i]).store(r, cuda::memory_order_relaxed);
     }
 }
 

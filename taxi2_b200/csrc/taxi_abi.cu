@@ -173,6 +173,8 @@ struct taxi_ctx {
     HostBuf<double> h_within_metrics;
     int64_t within_total = 0;
     bool within_held = false;
+    // taxi_clusters_within: the union-find forests of one call ([nthresholds][n]), not carried between calls
+    DevBuf<int32_t> d_forest;
     // stats of the last call
     int64_t launches = 0, cells = 0;
     double kernel_ms = 0.0;
@@ -699,6 +701,7 @@ void taxi_ctx_destroy(taxi_ctx* c)
     c->d_redo.release(); c->d_redo_count.release(); c->d_rscore.release(); c->d_rcounts.release(); c->d_rmetrics.release(); c->d_argidx.release(); c->d_argval.release(); c->d_bestcounts.release(); c->d_bestmetrics.release();
     c->d_rowcnt.release(); c->d_rowoff.release(); c->d_scantmp.release();
     c->h_within_idx.release(); c->h_within_counts.release(); c->h_within_metrics.release();
+    c->d_forest.release();
     cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1);
     cudaStreamDestroy(c->stream);
     delete c;
@@ -1624,6 +1627,73 @@ int taxi_pairs_within_fetch(taxi_ctx* c, int32_t* out_index, double* out_metrics
     std::memcpy(out_index, c->h_within_idx.p, n * sizeof(int32_t));
     if (out_metrics) std::memcpy(out_metrics, c->h_within_metrics.p, n * 4 * sizeof(double));
     if (out_counts) std::memcpy(out_counts, c->h_within_counts.p, n * 4 * sizeof(int32_t));
+    return TAXI_OK;
+}
+
+static_assert(TAXI_CLUSTER_MAX_THRESHOLDS == CLUSTER_MAX_THRESHOLDS, "header and kernel agree on the threshold limit");
+
+int taxi_clusters_within(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int32_t ny, int32_t metric, int32_t align,
+                         const double* thresholds, int32_t nthresholds, double scale, const int32_t* seed, int32_t* out_label)
+{
+    int rc = check_ctx(c, align != 0);
+    if (rc) return rc;
+    reset_stats(c);
+    if (c->set[1].loaded) return fail(TAXI_E_ARG, "clusters are of set 0 against itself, and set 1 is loaded");
+    if (metric < 0 || metric > 3 || !thresholds || !out_label) return fail(TAXI_E_ARG, "bad argument");
+    if (nthresholds < 1 || nthresholds > TAXI_CLUSTER_MAX_THRESHOLDS)
+        return fail(TAXI_E_ARG, "%d thresholds, outside 1..%d", nthresholds, TAXI_CLUSTER_MAX_THRESHOLDS);
+    for (int32_t t = 0; t < nthresholds; ++t)
+        if (std::isnan(thresholds[t])) return fail(TAXI_E_ARG, "threshold %d is NaN", t);
+    if (!std::isfinite(scale) || !(scale > 0.0)) return fail(TAXI_E_ARG, "scale %g is not finite and positive", scale);
+    if ((rc = check_rect(c, x0, nx, y0, ny))) return rc;
+    if (ny == 0) return fail(TAXI_E_ARG, "no columns to link");
+    const long long chunk = align ? kChunkPairs : kCountChunkPairs;
+    if (ny > chunk) return fail(TAXI_E_ARG, "too many columns for one device block (%d > %lld)", ny, chunk);
+    const int32_t n = c->set[0].n;
+    const size_t total = (size_t)nthresholds * n;
+    // the forests start from the seed's components (every node hooked straight under its label, the
+    // component's minimum) or from singletons; out_label stages them on the way to the device
+    if (seed) {
+        for (int32_t t = 0; t < nthresholds; ++t) {
+            const int32_t* s = seed + (size_t)t * n;
+            for (int32_t i = 0; i < n; ++i)
+                if (s[i] < 0 || s[i] > i || s[s[i]] != s[i])
+                    return fail(TAXI_E_ARG, "seed[%d][%d] = %d is not a canonical label (the smallest index of its component)", t, i, s[i]);
+        }
+        if (seed != out_label) std::memcpy(out_label, seed, total * sizeof(int32_t));
+    } else {
+        for (size_t k = 0; k < total; ++k) out_label[k] = (int32_t)(k % (size_t)n);
+    }
+    if (nx == 0) return TAXI_OK;
+    ON_DEVICE(c->device);
+    const int32_t rows = (int32_t)std::max<long long>(1, std::min<long long>(nx, chunk / ny));
+    const uint32_t flags = TAXI_OUT_METRICS;   // only the metric column takes part
+    if ((rc = reserve_outputs(c, (long long)rows * ny, flags))) return rc;
+    CUDA_TRY(c->d_forest.reserve(total));
+    CUDA_TRY(cudaMemcpyAsync(c->d_forest.p, out_label, total * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+    LinkArgs a{};
+    a.ny = ny; a.metric = metric; a.scale = scale; a.y0 = y0; a.n = n; a.parent = c->d_forest.p;
+    for (int32_t t = 0; t < nthresholds; ++t) a.threshold[t] = thresholds[t];
+    for (int u = 0; u < WITHIN_STEPS; ++u) a.live |= ((1u << nthresholds) - 1u) << (CLUSTER_MAX_THRESHOLDS * u);
+    const int wpb = 8;
+    for (int32_t r0 = 0; r0 < nx; r0 += rows) {
+        const int32_t nr = std::min(rows, nx - r0);
+        if (align) rc = taxi_align_rect_device(c, x0 + r0, nr, y0, ny, flags, nullptr, nullptr, c->d_metrics.p);
+        else rc = taxi_count_rect_device(c, x0 + r0, nr, y0, ny, flags, nullptr, c->d_metrics.p);
+        if (rc) return rc;
+        a.metrics = c->d_metrics.p; a.nx = nr; a.x0 = x0 + r0;
+        link_within_kernel<<<(nr + wpb - 1) / wpb, wpb * 32, 0, c->stream>>>(a);
+        CUDA_TRY(cudaGetLastError());
+        c->launches += 1;
+        if ((rc = finish_align(c))) return rc;
+    }
+    const int threads = 256;
+    const dim3 grid((unsigned)std::min<long long>((n + threads - 1) / threads, 4LL * c->sms), (unsigned)nthresholds);
+    flatten_kernel<<<grid, threads, 0, c->stream>>>(c->d_forest.p, n);
+    CUDA_TRY(cudaGetLastError());
+    c->launches += 1;
+    CUDA_TRY(cudaMemcpyAsync(out_label, c->d_forest.p, total * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
     return TAXI_OK;
 }
 

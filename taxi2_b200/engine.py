@@ -342,6 +342,25 @@ class Engine:
         N.check(self._lib.taxi_pairs_within_fetch(self._ctx, _p(index), _p(metrics), _p(counts)))
         return dict(row_ptr=row_ptr, index=index, metrics=metrics, counts=counts)
 
+    def clusters_within(self, x0: int, nx: int, y0: int, ny: int, thresholds, metric: int = 0, align: bool = True,
+                        scale: float = 1.0, seed: np.ndarray | None = None) -> np.ndarray:
+        """Single-linkage clusters of set 0 at one or more thresholds (taxi_clusters_within): x and y
+        are linked at threshold t iff the pair (x, y) of rows x0..x0+nx x columns [y0, y0+ny) of set 0
+        x set 0 has a value v of metric column `metric` that is not NaN and v * scale <= t (the
+        predicate of pairs_within); the pairs (i, i) link nothing.  Returns labels (m, n) int32 for
+        the m thresholds (a float or a sequence of up to 8) and the n sequences of set 0: the smallest
+        index in each sequence's component.  seed, an earlier result of the same shape, starts the
+        components from its labeling, so calls over disjoint row ranges chain."""
+        ts = np.ascontiguousarray(np.atleast_1d(np.asarray(thresholds, dtype=np.float64)).ravel())
+        labels = np.empty((len(ts), self.n[0]), dtype=np.int32)
+        if seed is not None:
+            seed = np.ascontiguousarray(seed, dtype=np.int32)
+            if seed.shape != labels.shape:
+                raise ValueError(f"seed must have shape {labels.shape} (thresholds x sequences of set 0), not {seed.shape}")
+        N.check(self._lib.taxi_clusters_within(self._ctx, x0, nx, y0, ny, int(metric), int(bool(align)), _p(ts), len(ts),
+                                               float(scale), _p(seed), _p(labels)))
+        return labels
+
     def best_matches(self, metric: int = 0, align: bool = True, rows_per_tile: int | None = None) -> dict:
         """versusReference at scale (BASELINE config C4): best_rows over all of set 0 x all of set 1."""
         return self.best_rows(0, self.n[0], 0, self.ny, metric, align)

@@ -11,7 +11,8 @@ Every pair is independent, so the pair matrix shards with no collective on the d
   one (page-locked) host array, or -- for the best-match row reduction of
   versus_reference.py:184-188 -- only the per-query winners (or k closest references) come back
   and column tiles of one query are combined on the host with the first-index tie-break; the
-  pairs within a threshold come back as per-tile CSR pieces, assembled on the host.
+  pairs within a threshold come back as per-tile CSR pieces, assembled on the host; clusters within
+  a threshold come back as one labeling per GPU, merged on the host.
 
 ctypes releases the GIL for the duration of a native call, so the threads really run concurrently;
 a context is only ever touched by its own thread while a run is in flight.
@@ -422,6 +423,38 @@ class MultiEngine:
         out.update(kernel_ms=kernel_ms, cells=cells, launches=launches, tiles=len(tiles))
         return out
 
+    def clusters_within(self, thresholds, metric: int = 0, align: bool = True, scale: float = 1.0,
+                        rows_per_tile: int | None = None, col_tiles: int = 1) -> dict:
+        """Single-linkage clusters of set 0 (loaded alone) at one or more thresholds over all of set 0
+        x set 0 (Engine.clusters_within).  Tiles are scheduled as in pairs_within (alignment-free: one or
+        two tiles per GPU unless rows_per_tile is given); every GPU chains
+        its own tiles through the seed, so it ends with one labeling of the links it computed, and
+        the labelings of the GPUs are merged here (combine_labels).  labels (m, n) int32, the
+        smallest index of every sequence's component per threshold, is the same for any tiling, tile
+        order and number of GPUs; clusters (m,) int64 counts the components."""
+        ts = np.atleast_1d(np.asarray(thresholds, dtype=np.float64)).ravel()
+        if rows_per_tile is None and not align:
+            # as in count_matrix: one or two tiles per GPU.  A union-find link waits on a chain of
+            # dependent loads, so the link kernel needs whole device blocks of rows to hide it
+            rows_per_tile = max(1, min(-(-self.nx // (2 * len(self.engines))), (1 << 26) // max(self.ny, 1)))
+        tiles = self.row_tiles(rows_per_tile, col_tiles)
+        own: dict[int, np.ndarray] = {}   # per context: the labeling of its tiles so far
+
+        def fn(engine: Engine, tile: Tile, slot: int):
+            key = id(engine)
+            own[key] = engine.clusters_within(tile.x0, tile.nx, tile.y0, tile.ny, ts, metric, align, scale, seed=own.get(key))
+            return engine.stats()
+
+        kernel_ms = cells = launches = 0
+        for _, st in self.run_tiles(tiles, fn, depth=4, ordered=False):
+            kernel_ms += st["kernel_ms"]; cells += st["cells"]; launches += st["launches"]
+        n = self.nx
+        labels = np.broadcast_to(np.arange(n, dtype=np.int32), (len(ts), n)).copy()
+        for lab in own.values():
+            labels = combine_labels(labels, lab)
+        clusters = (labels == np.arange(n, dtype=np.int32)).sum(axis=1, dtype=np.int64)
+        return dict(labels=labels, clusters=clusters, kernel_ms=kernel_ms, cells=cells, launches=launches, tiles=len(tiles))
+
 
 def _accumulate(acc: dict, engine, redo: bool) -> None:
     st = engine.stats()
@@ -507,3 +540,35 @@ def combine_within(tiles, nx: int) -> dict:
         counts[dst] = piece["counts"]
         fill[x0:x0 + n] += lens
     return dict(row_ptr=row_ptr, index=index, metrics=metrics, counts=counts)
+
+
+def combine_labels(a: np.ndarray, b: np.ndarray) -> np.ndarray:
+    """The canonical labeling of the union of two canonical labelings of the same nodes: nodes
+    together in a or in b are together in the result, and every node is labelled with the smallest
+    index of its merged component.  a and b have shape (..., n), label[i] <= i and
+    label[label[i]] == label[i] along the last axis (what clusters_within returns).  Each round
+    gives every node the smallest label over its group in a and its group in b, then the label of
+    that label; the minimum of a component spreads through it and the rounds stop when nothing
+    changes.  numpy only; commutative and associative, so any merge order gives the same array."""
+    a = np.asarray(a)
+    b = np.asarray(b)
+    if a.shape != b.shape:
+        raise ValueError(f"labelings of different shapes {a.shape} and {b.shape}")
+    n = a.shape[-1] if a.ndim else 0
+    if a.size == 0:
+        return np.empty(a.shape, dtype=np.int32)
+    # one flat node space: row r of the leading axes owns the indices r * n .. r * n + n
+    base = (np.arange(a.size // n, dtype=np.int64) * n)[:, None]
+    fa = (a.reshape(-1, n).astype(np.int64) + base).ravel()
+    fb = (b.reshape(-1, n).astype(np.int64) + base).ravel()
+    lab = np.minimum(fa, fb)
+    while True:
+        low = np.full(lab.size, lab.size, dtype=np.int64)
+        np.minimum.at(low, fa, lab)
+        np.minimum.at(low, fb, lab)
+        new = np.minimum(low[fa], low[fb])
+        new = np.minimum(new, new[new])
+        if np.array_equal(new, lab):
+            break
+        lab = new
+    return (lab.reshape(-1, n) - base).reshape(a.shape).astype(np.int32)

@@ -86,7 +86,9 @@ int taxi_align_rect(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t n
 /*
  * Device-resident variant used for kernel-only timing and by callers that keep results in HBM:
  * the out_* arguments are DEVICE pointers (e.g. torch tensors' data_ptr()), nothing is copied.
- * The work is enqueued on the context's stream; taxi_sync() waits for it.
+ * The work is enqueued on the context's stream; taxi_sync() waits for it.  Requested outputs must be
+ * aligned: d_score 4-byte, d_counts and d_metrics 16-byte (a pair's counts leave as one 128-bit store,
+ * its metrics as two); anything else is TAXI_E_ARG, checked before any work, nx * ny = 0 included.
  */
 int taxi_align_rect_device(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t ny, uint32_t flags,
                            int32_t* d_score, int32_t* d_counts, double* d_metrics);
@@ -99,7 +101,7 @@ int taxi_sync(taxi_ctx* ctx);
  * of (x, y); the first alignment differs only where Ix and Iy tie on the traced path, which the kernel
  * detects -- those pairs (taxi_last_redo() of them, 0.7 % of COI barcodes) are re-aligned the other
  * way round, the rest mirror their result.  Bit-identical to two taxi_align_rect_device calls.
- * Synchronous.
+ * Synchronous.  d_* and t_* follow the alignment rule of taxi_align_rect_device.
  */
 int taxi_align_rect_both_device(taxi_ctx* ctx, int32_t x0, int32_t nx, int32_t y0, int32_t ny, uint32_t flags,
                                 int32_t* d_score, int32_t* d_counts, double* d_metrics,
@@ -151,7 +153,9 @@ int taxi_count_pairs(taxi_ctx* ctx, const int32_t* px, const int32_t* py, int64_
 /*
  * Best match per query row (versus_reference.py:184-188, decontaminate.py:258-264): first minimum
  * of metric column `metric` (0..3) over each row of an nx x ny metrics matrix (device pointer,
- * 4 doubles per pair); NaN never wins.  out_index[x] = -1 when the whole row is undefined.
+ * 4 doubles per pair, 8-byte aligned, else TAXI_E_ARG); NaN never wins, equal values go to the smaller
+ * column.  out_index[x] = -1 and out_value[x] = NaN when the whole row is undefined; out_value_host may
+ * be NULL.  Host output pointers.
  */
 /*
  * The metric formulas on their own (distances.py:319-348 applied to counts instead of strings): n tuples

@@ -627,6 +627,15 @@ int reserve_outputs(taxi_ctx* c, int64_t n, uint32_t flags)
     return TAXI_OK;
 }
 
+// Caller-owned device outputs of the alignment kernels (and scatter_redo_kernel): a pair's counts
+// leave as one 128-bit store and its metrics as two; a misaligned pointer would fault on the device.
+int check_output_alignment(const int32_t* score, const int32_t* counts, const double* metrics)
+{
+    if (((uintptr_t)score & 3) || ((uintptr_t)counts & 15) || ((uintptr_t)metrics & 15))
+        return fail(TAXI_E_ARG, "d_score must be 4-byte, d_counts and d_metrics 16-byte aligned");
+    return TAXI_OK;
+}
+
 int download_outputs(taxi_ctx* c, int64_t n, uint32_t flags, int32_t* score, int32_t* counts, double* metrics)
 {
     if ((flags & TAXI_OUT_SCORE) && score)
@@ -805,6 +814,11 @@ int taxi_align_rect_device(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int3
     if (rc) return rc;
     c->within_held = false;
     if ((rc = check_rect(c, x0, nx, y0, ny))) return rc;
+    AlignArgs a{};
+    a.score = (flags & TAXI_OUT_SCORE) ? d_score : nullptr;
+    a.counts = (flags & TAXI_OUT_COUNTS) ? d_counts : nullptr;
+    a.metrics = (flags & TAXI_OUT_METRICS) ? d_metrics : nullptr;
+    if ((rc = check_output_alignment(a.score, a.counts, a.metrics))) return rc;
     ON_DEVICE(c->device);
     const long long npairs = (long long)nx * ny;
     if (npairs == 0) return TAXI_OK;
@@ -812,11 +826,7 @@ int taxi_align_rect_device(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0, int3
         return fail(TAXI_E_EMPTY, "sequence has zero length");
     const int mr = max_len_range(c->set[0], x0, nx), mc = max_len_range(yset(c), y0, ny);
     if ((rc = range_check(c, mr, mc))) return rc;
-    AlignArgs a{};
     fill_rect(a, c, x0, y0, ny, npairs);
-    a.score = (flags & TAXI_OUT_SCORE) ? d_score : nullptr;
-    a.counts = (flags & TAXI_OUT_COUNTS) ? d_counts : nullptr;
-    a.metrics = (flags & TAXI_OUT_METRICS) ? d_metrics : nullptr;
     c->cells += cells_rect(c->set[0], yset(c), x0, nx, y0, ny);
 
     // Columns of unequal length: a warp sweeps max(len_y) columns for its two pairs, so pairing a
@@ -987,6 +997,10 @@ int taxi_align_rect_both_device(taxi_ctx* c, int32_t x0, int32_t nx, int32_t y0,
     if (rc) return rc;
     c->within_held = false;
     if ((rc = check_rect(c, x0, nx, y0, ny))) return rc;
+    if ((rc = check_output_alignment((flags & TAXI_OUT_SCORE) ? d_score : nullptr, (flags & TAXI_OUT_COUNTS) ? d_counts : nullptr,
+                                     (flags & TAXI_OUT_METRICS) ? d_metrics : nullptr)) ||
+        (rc = check_output_alignment((flags & TAXI_OUT_SCORE) ? t_score : nullptr, (flags & TAXI_OUT_COUNTS) ? t_counts : nullptr,
+                                     (flags & TAXI_OUT_METRICS) ? t_metrics : nullptr))) return rc;
     ON_DEVICE(c->device);
     const long long npairs = (long long)nx * ny;
     if (npairs == 0) return TAXI_OK;
@@ -1441,6 +1455,7 @@ int taxi_argmin_rows_device(taxi_ctx* c, const double* d_metrics, int32_t nx, in
 {
     if (!c || !d_metrics || nx < 0 || ny <= 0 || metric < 0 || metric > 3 || !out_index_host)
         return fail(TAXI_E_ARG, "bad argument");
+    if ((uintptr_t)d_metrics & 7) return fail(TAXI_E_ARG, "d_metrics must be 8-byte aligned");
     c->within_held = false;
     if (nx == 0) return TAXI_OK;
     ON_DEVICE(c->device);

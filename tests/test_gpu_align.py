@@ -9,6 +9,7 @@ import pytest
 
 import oracle
 from conftest import GOLDEN
+from poison import poison
 from synth import coi_like, random_pairs, read_tab_sequences
 
 pytestmark = pytest.mark.gpu
@@ -426,6 +427,7 @@ def test_full_size_tile_properties(engine):
         engine.set_option("force_top", opts[1])
         try:
             engine.set_scores(None)
+            poison(engine, n * n, int(lens.max()) + 1)
             engine.load(seqs, 0)
             results[name] = engine.align_rect(0, n, 0, n)
             results[name]["kernel"] = engine.last_kernel

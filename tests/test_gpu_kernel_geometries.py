@@ -24,6 +24,7 @@ import pytest
 import kernel_geometry as K
 import oracle
 import packed16_rule as R
+from poison import poison
 from synth import ALPHA, coi_like, random_pairs
 from test_gpu_packed_exactness import assert_metrics_close, oracle_batch
 
@@ -233,6 +234,7 @@ def run_pairs(engine, xs, ys, scores, opts, family, H, strings=True):
     want = oracle_batch(xs, ys, px, px, scores)
     with Options(engine, **opts):
         engine.set_scores(scores)
+        poison(engine, n, max(la + lb) + 1)
         engine.load(xs, 0)
         engine.load(ys, 1)
         got = engine.align_pairs(px, px)
@@ -274,6 +276,9 @@ def test_intra_task_stripe_counts(engine, case):
     assert K.instance(case["scores"], la, lb, "pairs", {"force_general": 1, "no_coop": 1})[0] == "general"
     px = np.arange(len(xs), dtype=np.int32)
     with Options(engine, force_general=1, no_coop=1):
+        poison(engine, len(xs), max(la + lb) + 1)
+        engine.load(xs, 0)
+        engine.load(ys, 1)
         ref = engine.align_pairs(px, px)
         assert engine.last_kernel == 32
     assert np.array_equal(got["score"], ref["score"]) and np.array_equal(got["counts"], ref["counts"])
@@ -290,6 +295,7 @@ def check_both(engine, xs, ys, H, tie_rich):
     la, lb = [len(x) for x in xs], [len(y) for y in ys]
     assert K.instance(DEFAULT, la, lb, "both") == ("both", H, 1)
     engine.set_scores(DEFAULT)
+    poison(engine, 2 * len(xs) * len(ys), max(la + lb) + 1)     # both halves: (x, y) and the mirrored (y, x)
     engine.load(xs, 0)
     if ys is not xs:
         engine.load(ys, 1)
